@@ -2,6 +2,7 @@
 """bench.py -- PAAC env-steps/sec (Nature CNN, t_max=5) on N B200s; update ms.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--envs E] [--math fp32|tf32x3|tf32]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -13,6 +14,10 @@ synthetic raw 210x160 frames, NatureNetwork, 4096 envs per GPU, t_max = 5, 6 act
 One step = 20,480 env-steps per GPU.  `value` = env-steps of all ranks / max-over-ranks device time with the
 frames resident in HBM; `e2e` = the same cycle driven from HOST buffers (pinned frames uploaded and sampled
 actions read back every env step, loss read back every update).  Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR: right after the K timed steps of the headline, rank 0 writes what the last of them computed as
+DIR/<name>.npy (float32; see dump_outputs()).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 
 --impl reference times the CPU restatement of the reference's path (oracle/cpu_baseline.py; TF1/ALE cannot be
 installed here) on the host cores for the same metric/config, each step a bounded sample of the workload.
@@ -58,7 +63,13 @@ def parse():
     ap.add_argument('--dev_slices', type=int, default=1,
                     help='device-resident arm: contiguous environment slices, each rolled out on its own stream (1 = whole batch on one stream)')
     ap.add_argument('--ref_envs', type=int, default=64, help='--impl reference: envs per step (bounded sample)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed to DIR/<name>.npy (float32, under 64 MB in all)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the B200 arm')
     if args.math == 'auto':
         args.math = 'bf16x3'
     return args
@@ -276,6 +287,39 @@ def bind_to_gpu_numa_node(local):
     return 0
 
 
+DUMP_ENVS = 4096            # --dump-outputs: per-environment outputs of at most this many environments (a seeded sample)
+DUMP_STATE_ENVS = 16        # and the preprocessed observations (28,224 B per environment and env step) of this many
+
+
+def dump_outputs(eng, out_dir):
+    """Write what the last update cycle of `eng` hands its caller to out_dir/<name>.npy as float32 (per-step arrays as
+    [T, n, ...]).  The n environments are a fixed seeded sample (env_index.npy), so the files stay under 64 MB at any --envs:
+    about 1.5 MB of per-environment outputs, 9 MB of observations and 20 MB of parameters, gradient and RMSProp slot
+    (Nature, 6 actions)."""
+    import numpy as np
+    import torch
+    T, N = eng.T, eng.N
+    pick = np.sort(np.random.RandomState(0).choice(N, min(N, DUMP_ENVS), replace=False))
+    spick = pick[np.sort(np.random.RandomState(1).choice(len(pick), min(len(pick), DUMP_STATE_ENVS), replace=False))]
+    idx, sidx = torch.from_numpy(pick).to(eng.dev), torch.from_numpy(spick).to(eng.dev)
+    per_step = lambda x: x.reshape((T, N) + x.shape[1:])[:, idx]
+    # the T observations of the rollout just trained on: s_1 .. s_{T-1} in the half update() rolled away from, s_T in slot 0
+    # of the current half
+    observed = torch.cat([eng._sbuf[1 - eng._cur, 1:], eng.state(0)[None]])[:, sidx]
+    out = {'env_index': idx, 'observed_states': observed,
+           'actions': eng.actions[:, idx], 'values': eng.values[:, idx], 'bootstrap_values': eng.boot_v[idx],
+           'pi': per_step(eng.pi), 'v': per_step(eng.v), 'returns': per_step(eng.y), 'advantages': per_step(eng.adv),
+           'dlogits': per_step(eng.dlogits), 'dv': per_step(eng.dv),
+           'loss': eng.loss, 'global_norm': eng.norm, 'grads': eng.grads, 'params': eng.net.params, 'rmsprop_ms': eng.ms}
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in out.items():
+        a = t.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+        total += a.nbytes
+    return {'dir': out_dir, 'arrays': len(out), 'bytes': total, 'envs_sampled': len(pick), 'state_envs_sampled': len(sidx)}
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -379,6 +423,7 @@ def run_b200(args):
     ms_plain = timed(step_device, args.steps)
     clk = clocks.stop()
     launches = net.launch_count() - launches0
+    dumped = dump_outputs(eng, args.dump_outputs) if args.dump_outputs and rank == 0 else None
     ms_per_step = ms_plain / args.steps
     value = world * N * T * args.steps / (ms_plain / 1e3)
     # pass 2 -- the same K steps with every kernel bracketed by a CUDA event pair on the launching stream (the per-kernel
@@ -614,6 +659,8 @@ def run_b200(args):
                 'profiled_ms_per_step': ms_total / args.steps,
                 'kernels': [{k: (round(v, 6) if isinstance(v, float) else v) for k, v in kk.items()} for kk in kernels],
                 'loss': loss_val}
+        if dumped:
+            line['dumped_outputs'] = dumped
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()

@@ -67,15 +67,6 @@ int paacb_get_math(const paacb_ctx* ctx);
 /* Multi-GPU: leave n_sms SMs free of the persistent conv weight-gradient CTAs (PAACB_BWD_HEAD), the kernels that run
  * while the caller's collective reduces the gradient tail, so that the collective's CTAs can be scheduled beside them. */
 int paacb_set_sm_reserve(paacb_ctx* ctx, int n_sms);
-/* bf16-split mode, OPT-IN (off by default: measured slower than one launch per layer on B200, DESIGN.md 3.3): the forward of a
- * batch (conv1 ... hidden fc) as ONE persistent kernel whose CTAs are partitioned between the layers; each layer reads what
- * the layer above wrote a few tiles earlier out of L2 (csrc/tc2_pipe.cu).  Results are bit-identical to the layer-by-layer
- * forward.  enable = 0: one launch per layer (the default); ctas_conv1/2/3 > 0
- * override the role sizes (the fc layer takes the remaining SMs; NIPS ignores ctas_conv3).  The hand-off counters are
- * context-owned, one set per stream that calls a forward (at most 4 streams; further streams run layer by layer).
- * paacb_forward_pipeline_errors: *out != 0 if a bounded hand-off wait ever gave up (synchronises; tests only). */
-int paacb_set_forward_pipeline(paacb_ctx* ctx, int enable, int ctas_conv1, int ctas_conv2, int ctas_conv3);
-int paacb_forward_pipeline_errors(const paacb_ctx* ctx, uint32_t* out);
 /* The tensor-core modes keep operand images of the parameters (bf16 hi/lo transposes, int8 digits of conv1) in the
  * context and reuse them across forwards of the same d_params pointer: PAAC runs t_max + 2 forwards per parameter
  * update.  paacb_clip_rmsprop refreshes the images itself; a caller that writes the parameter buffer by any other

@@ -24,8 +24,6 @@ PROTOTYPES = {
     'paacb_set_math': (_i, [_vp, _i]),
     'paacb_get_math': (_i, [_vp]),
     'paacb_set_sm_reserve': (_i, [_vp, _i]),
-    'paacb_set_forward_pipeline': (_i, [_vp, _i, _i, _i, _i]),
-    'paacb_forward_pipeline_errors': (_i, [_vp, C.POINTER(C.c_uint32)]),
     'paacb_set_resize_tables': (_i, [_vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     'paacb_param_count': (_i64, [_vp]),
     'paacb_num_tensors': (_i, [_vp]),

@@ -194,69 +194,17 @@ int paacb_create(paacb_ctx** out, int arch, int num_actions, int device) {
       cudaGetLastError();
       c->opt_counter = nullptr;          // falls back to the two-launch optimizer
     }
-    // hand-off counters of the layer-pipelined forward (tc2_pipe.cu): per buffer 2 counters per sample + 2 per 128 samples
-    c->pipe_buf_words = (size_t)(2 * paacb_ctx::kPipeMaxBatch + 2 * (paacb_ctx::kPipeMaxBatch / 128 + 2));
-    if (cudaMalloc(&c->pipe_cnt, (paacb_ctx::kPipeBufs * c->pipe_buf_words + 64) * sizeof(uint32_t)) == cudaSuccess) {
-      c->pipe_err = c->pipe_cnt + paacb_ctx::kPipeBufs * c->pipe_buf_words;
-      cudaMemset(c->pipe_err, 0, 64 * sizeof(uint32_t));
-    } else {
-      cudaGetLastError();
-      c->pipe_cnt = nullptr;             // the forward stays layer by layer
-      c->pipe_err = nullptr;
-    }
     cudaSetDevice(cur);
   }
   {
-    // The layer-pipelined forward is OPT-IN (PAACB_PIPE=1 or paacb_set_forward_pipeline): measured on B200 it is bit-identical
-    // but 13-60 % SLOWER than one launch per layer (profiles/r02_pipe_tune.json; DESIGN.md section 3.3 says why), so the
-    // product path launches the layers one by one.  Role sizes: CTAs of conv1 / conv2 / conv3 out of the device's SMs, the fc
-    // layer takes the rest; PAACB_PIPE_SPLIT="a,b,c" overrides the split, PAACB_PIPE_MIN_BATCH the smallest batch that uses it.
     const char* c3 = getenv("PAACB_CONV3_PACKED");
     c->conv3_packed = (c3 != nullptr) ? atoi(c3) : 1;
     const char* rk = getenv("PAACB_SM_RESERVE_KERNELS");
     c->sm_reserve_kernels = (rk != nullptr) ? atoi(rk) : 3;
     const char* e = getenv("PAACB_PDL");
     c->pdl_on = (e == nullptr) ? 1 : atoi(e);
-    e = getenv("PAACB_PIPE");
-    c->pipe_on = (e == nullptr) ? 0 : atoi(e);
-    e = getenv("PAACB_PIPE_MIN_BATCH");
-    c->pipe_min_batch = (e == nullptr) ? 1 : atoll(e);
-    const double f1 = arch == PAACB_ARCH_NATURE ? 0.30 : 0.45, f2 = arch == PAACB_ARCH_NATURE ? 0.28 : 0.30,
-                 f3 = arch == PAACB_ARCH_NATURE ? 0.23 : 0.0;
-    c->pipe_split[0] = (int)(f1 * c->num_sms + 0.5);
-    c->pipe_split[1] = (int)(f2 * c->num_sms + 0.5);
-    c->pipe_split[2] = (int)(f3 * c->num_sms + 0.5);
-    e = getenv("PAACB_PIPE_SPLIT");
-    if (e != nullptr) {
-      int a = 0, b = 0, d = 0;
-      if (sscanf(e, "%d,%d,%d", &a, &b, &d) >= 2) { c->pipe_split[0] = a; c->pipe_split[1] = b; c->pipe_split[2] = d; }
-    }
   }
   *out = c;
-  return PAACB_OK;
-}
-
-int paacb_set_forward_pipeline(paacb_ctx* ctx, int enable, int ctas_conv1, int ctas_conv2, int ctas_conv3) {
-  PAACB_CHECK_ARG(ctx != nullptr, "ctx is NULL");
-  PAACB_CHECK_ARG(ctas_conv1 >= 0 && ctas_conv2 >= 0 && ctas_conv3 >= 0 && ctas_conv1 + ctas_conv2 + ctas_conv3 < ctx->num_sms,
-                  "the role sizes must leave at least one SM to the fc layer");
-  ctx->pipe_on = enable ? 1 : 0;
-  if (ctas_conv1 > 0 && ctas_conv2 > 0) {
-    ctx->pipe_split[0] = ctas_conv1;
-    ctx->pipe_split[1] = ctas_conv2;
-    ctx->pipe_split[2] = ctas_conv3;
-  }
-  return PAACB_OK;
-}
-
-int paacb_forward_pipeline_errors(const paacb_ctx* ctx, uint32_t* out) {
-  PAACB_CHECK_ARG(ctx != nullptr && out != nullptr, "NULL argument");
-  *out = 0u;
-  if (ctx->pipe_err == nullptr) return PAACB_OK;
-  if (cudaMemcpy(out, ctx->pipe_err, sizeof(uint32_t), cudaMemcpyDeviceToHost) != cudaSuccess) {
-    set_error("paacb_forward_pipeline_errors: %s", cudaGetErrorString(cudaGetLastError()));
-    return PAACB_ECUDA;
-  }
   return PAACB_OK;
 }
 
@@ -268,7 +216,6 @@ int paacb_destroy(paacb_ctx* ctx) {
     delete[] ctx->prof_kid;
   }
   if (ctx->opt_counter != nullptr) cudaFree(ctx->opt_counter);
-  if (ctx->pipe_cnt != nullptr) cudaFree(ctx->pipe_cnt);
   if (ctx->wpack_hi != nullptr) cudaFree(ctx->wpack_hi);
   if (ctx->wpack_lo != nullptr) cudaFree(ctx->wpack_lo);
   if (ctx->wpack_d_hi != nullptr) cudaFree(ctx->wpack_d_hi);
@@ -322,7 +269,6 @@ int paacb_profile_read(const paacb_ctx* ctx, int slot, char* name, int name_cap,
     else if (slot < K_SUMSQ) { base = "dgrad"; layer = slot - K_DGRAD0; }
     else if (slot == K_SUMSQ) base = "grad_sumsq";
     else if (slot == K_RMSPROP) base = "clip_rmsprop";
-    else if (slot == K_FWD_PIPE) base = "forward_pipe";
     else base = "pack_weights";
     if (layer >= 0) {
       if (layer < ctx->n_layers) {
@@ -574,13 +520,8 @@ static int forward_impl(const paacb_ctx* ctx, const float* d_params, const uint8
   if (rc != PAACB_OK) return rc;
   if (ctx->math == PAACB_MATH_BF16X3) {
     const int L = ctx->n_layers;
-    // conv1 ... fc: one layer-pipelined persistent kernel (tc2_pipe.cu) or, where that does not apply, layer by layer
-    rc = launch_forward_pipe_bf16(ctx, d_params, d_states, d_fwd_ws, batch, slice, st);
-    if (rc == PAACB_EUNSUPPORTED) {
-      rc = PAACB_OK;
-      for (int l = 0; l < L - 1 && rc == PAACB_OK; ++l) rc = launch_conv_fwd_bf16(ctx, l, d_params, d_states, d_fwd_ws, batch, slice, st);
-      if (rc == PAACB_OK) rc = launch_fc_fwd_bf16(ctx, L - 1, d_params, d_fwd_ws, batch, slice, st);
-    }
+    for (int l = 0; l < L - 1 && rc == PAACB_OK; ++l) rc = launch_conv_fwd_bf16(ctx, l, d_params, d_states, d_fwd_ws, batch, slice, st);
+    if (rc == PAACB_OK) rc = launch_fc_fwd_bf16(ctx, L - 1, d_params, d_fwd_ws, batch, slice, st);
     if (rc != PAACB_OK) return rc;
     const Planes hp = layer_planes(d_fwd_ws, ctx->layer[L - 1].out_act_off, ctx->feat, slice);
     return launch_heads_fwd(ctx, nullptr, reinterpret_cast<const uint16_t*>(hp.hi), reinterpret_cast<const uint16_t*>(hp.lo),

@@ -53,7 +53,7 @@ struct ResizeTables {
 // profiling slots: one per kernel family per layer (paacb_profile_read)
 enum KernelId {
   K_PREPROCESS = 0, K_FWD0 = 1, K_HEADS_FWD = 5, K_LOSS = 6, K_HEADS_BWD = 7, K_WGRAD0 = 8, K_DGRAD0 = 12,
-  K_SUMSQ = 16, K_RMSPROP = 17, K_PACK = 18, K_FWD_PIPE = 19, K_COUNT = 20
+  K_SUMSQ = 16, K_RMSPROP = 17, K_PACK = 18, K_COUNT = 19
 };
 constexpr int kMaxProfEvents = 8192;
 
@@ -131,17 +131,6 @@ struct paacb_ctx {
                                 // copy pipeline, 2 = pinned host frames too (on k1_pipe_host_grid CTAs: PCIe needs few loads in flight)
   int k1_pipe_host_grid;        // PAACB_K1_PIPE_HOST_GRID (default 32)
   int k1_hints;                 // PAACB_K1_HINTS (default 3): bit 0 = inputs read evict-first, bit 1 = new stack written evict-last
-  // layer-pipelined forward (tc2_pipe.cu): hand-off counters (one buffer per stream in use), role sizes, sticky error word
-  static constexpr int kPipeBufs = 4;
-  static constexpr int64_t kPipeMaxBatch = 32768;
-  int pipe_on;                  // paacb_set_forward_pipeline / PAACB_PIPE
-  int64_t pipe_min_batch;       // batches below this use the layer-by-layer forward
-  int pipe_split[3];            // CTAs of conv1, conv2, conv3 (the fc layer takes the rest of the SMs)
-  uint32_t* pipe_cnt;           // kPipeBufs buffers of pipe_buf_words words
-  size_t pipe_buf_words;
-  uint32_t* pipe_err;
-  mutable int pipe_nbuf;
-  mutable void* pipe_stream[kPipeBufs];
   int conv3_packed;             // PAACB_CONV3_PACKED (default 1): conv3 forward with two whole samples per tile (tc2_conv.cuh: Geo<G_FWD3P>)
   int pdl_on;                   // PAACB_PDL (default 1): programmatic dependent launch between the kernels of one forward / backward
   int sm_reserve_kernels;       // PAACB_SM_RESERVE_KERNELS (default 3): how many of the conv weight-gradient kernels, in launch order, leave them
@@ -248,12 +237,6 @@ int launch_clip_rmsprop(const paacb_ctx* ctx, float* params, float* ms, float* m
                         float* norm_out, float* ws, cudaStream_t st);
 
 int launch_grad_stats(const paacb_ctx* ctx, const float* grads, float gscale, float* ws, double* out4, cudaStream_t st);
-
-// layer-pipelined forward of the bf16-split path (tc2_pipe.cu): conv1 ... fc in one persistent kernel; PAACB_EUNSUPPORTED:
-// not enabled / not applicable, the caller launches the layers one by one
-struct WsSlice;
-int launch_forward_pipe_bf16(const paacb_ctx* ctx, const float* params, const uint8_t* states, void* fwd_ws, int64_t batch,
-                             const WsSlice& slice, cudaStream_t st);
 
 // tcgen05 path (gemm_tc.cu); returns PAACB_EUNSUPPORTED when a layer/mode is not covered
 int launch_pack_weights(const paacb_ctx* ctx, const LayerGeom& g, const float* w, cudaStream_t st);

@@ -207,9 +207,8 @@ static int weight_maps(const paacb_ctx* ctx, const uint16_t* hi, const uint16_t*
   return encode_tmap_bf16(&out[1], lo + g.w_off, 2, dims, strides, box, 128);
 }
 
-// prep != nullptr: fill *prep and *prep_geo (the Geo<> id of the layer) instead of launching (tc2_pipe.cu)
-static int conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const uint8_t* states, void* fwd_ws, int64_t batch,
-                         const WsSlice& slice, cudaStream_t st, ConvKParams* prep, int* prep_geo) {
+int launch_conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const uint8_t* states, void* fwd_ws, int64_t batch,
+                         const WsSlice& slice, cudaStream_t st) {
   const LayerGeom& g = ctx->layer[l];
   ConvKParams p;
   memset(&p, 0, sizeof(p));
@@ -249,14 +248,9 @@ static int conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const
     const int64_t q_total = batch * Ge::HQ * Ge::WU;                                                               \
     if (q_total >= (1LL << 31) - 256) return PAACB_EUNSUPPORTED;                                                   \
     p.num_tiles = (int)((q_total + 127) / 128);                                                                    \
-    if (prep != nullptr) {                                                                                         \
-      *prep = p;                                                                                                   \
-      *prep_geo = GE;                                                                                              \
-      return PAACB_OK;                                                                                             \
-    }                                                                                                              \
     return launch_convk<GE>(ctx, p, K_FWD0 + l, st);                                                               \
   }
-  if (l == 0) return prep != nullptr ? PAACB_EUNSUPPORTED : launch_conv1_fwd_i8(ctx, params, states, fwd_ws, batch, slice, st);
+  if (l == 0) return launch_conv1_fwd_i8(ctx, params, states, fwd_ws, batch, slice, st);
   // (each case leaves its do-while with `break` when the layer's geometry is not the one it was written for)
   if (l == 1) do PAACB_FWD_CASE(G_FWD2) while (0);
   if (l == 1) do PAACB_FWD_CASE(G_FWD2N) while (0);
@@ -276,25 +270,11 @@ static int conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const
     if (rc == PAACB_OK) rc = weight_maps(ctx, ctx->wb_f_hi, ctx->wb_f_lo, g, (uint64_t)g.K, (uint64_t)g.N, Ge::BN, p.tmW);
     if (rc != PAACB_OK) return rc;
     p.num_tiles = (int)((batch + GeoPack<G_FWD3P>::SAMPLES - 1) / GeoPack<G_FWD3P>::SAMPLES);
-    if (prep != nullptr) {
-      *prep = p;
-      *prep_geo = G_FWD3P;
-      return PAACB_OK;
-    }
     return launch_convk<G_FWD3P>(ctx, p, K_FWD0 + l, st);
   } while (0);
   if (l == 2) do PAACB_FWD_CASE(G_FWD3) while (0);
 #undef PAACB_FWD_CASE
   return PAACB_EUNSUPPORTED;
-}
-
-int launch_conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const uint8_t* states, void* fwd_ws, int64_t batch,
-                         const WsSlice& slice, cudaStream_t st) {
-  return conv_fwd_bf16(ctx, l, params, states, fwd_ws, batch, slice, st, nullptr, nullptr);
-}
-int prepare_conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, void* fwd_ws, int64_t batch, const WsSlice& slice,
-                          ConvKParams* p, int* geo) {
-  return conv_fwd_bf16(ctx, l, params, nullptr, fwd_ws, batch, slice, nullptr, p, geo);
 }
 
 // dX of layer l's input: A = dZ planes of layer l (bwd_ws), output = dZ planes of layer l-1, masked by layer l-1's activation

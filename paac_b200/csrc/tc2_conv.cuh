@@ -1,8 +1,7 @@
-// Patch-resident implicit GEMMs of the conv layers (forward and data gradient): geometry, parameters and the kernel body
-// (shared by the stand-alone kernels of tc2_conv.cu and the layer-pipelined forward of tc2_pipe.cu).  Design: tc2_conv.cu.
+// Patch-resident implicit GEMMs of the conv layers (forward and data gradient): geometry, parameters and the kernel.
+// Design: tc2_conv.cu.
 #pragma once
 #include "tc2.cuh"
-#include "tc2_pipe.cuh"
 
 namespace paacb {
 
@@ -169,15 +168,14 @@ __device__ __forceinline__ float warp_transpose_sum(float (&v)[32], int lane) {
   return v[0];
 }
 
-// cta / ncta: this CTA's index and count among the CTAs that run this layer.  PIPE (forward only): the TMA producer waits for
-// the samples a tile reads to be complete in the layer above, the epilogue signals the samples it completed (tc2_pipe.cuh).
-template <int G, bool PIPE>
-__device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, const int ncta, uint8_t* smem_raw, const PipeIO& io) {
+template <int G>
+__global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __grid_constant__ ConvKParams p) {
+  const int cta = (int)blockIdx.x, ncta = (int)gridDim.x;   // persistent CTAs: this one's index, their count
   using Ge = Geo<G>;
   using Cfg = ConvKCfg<G>;
   constexpr int NSLOTS = Ge::NSLOTS, BN = Ge::BN, NACC = Ge::NACC;
-  static_assert(!PIPE || !Ge::DGRAD, "the pipelined hand-off is a forward feature");
   constexpr int PACK = GeoPack<G>::SAMPLES;       // > 0: whole samples per tile, one patch copy per filter row
+  extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* ring = smem;
   uint8_t* wsm = smem + Cfg::RING_BYTES;
@@ -233,15 +231,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
       int slot = 0;
       uint32_t phase = 0;
       for (int tile = cta; tile < p.num_tiles; tile += ncta) {
-        if constexpr (PIPE) {
-          // the tile's positions [128 tile, 128 tile + 128) belong to these samples of the layer above (WU * HQ positions each);
-          // rows the box reads beyond them feed only positions that are discarded
-          constexpr int PPS = Ge::WU * Ge::HQ;
-          const int n0 = PACK > 0 ? PACK * tile : (tile * 128) / PPS;
-          int n1 = PACK > 0 ? PACK * tile + PACK - 1 : (tile * 128 + 127) / PPS;
-          if (n1 > p.batch - 1) n1 = p.batch - 1;
-          pipe_wait(io, n0, n1, io.up_target);
-        }
         // (requesting the boxes of the tile after next into L2 with cp.async.bulk.prefetch.tensor was measured: 3 % slower; the
         // packed conv3 geometry with the NEXT tile's two samples prefetched: 0.603 -> 0.617 ms per step, tools/gpu_round2_x.sh;
         // prefetch.global.L2 of the tile after next by the idle epilogue threads, one per 128-byte line: conv2 0.76-0.79 -> 0.79-0.83,
@@ -452,7 +441,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
     float bsum[NACC == 1 ? BN / 32 : 1];
 #pragma unroll
     for (int i = 0; i < (NACC == 1 ? BN / 32 : 1); ++i) bsum[i] = 0.f;
-    PipeNote note = pipe_note_none();
     for (int tl = grp, tile = cta + grp * ncta; tile < p.num_tiles; tile += 2 * ncta, tl += 2) {
       const int ab = grp;
       const uint32_t aph = (uint32_t)((tl >> 1) & 1);
@@ -460,7 +448,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
       bool ok;
       int64_t pix = 0;          // forward: output pixel index; dgrad: (sample, qh, qw) resolved per class below
       int qh = 0, qw = 0;
-      int n_fwd = 0;            // forward: sample of this row
       if constexpr (Ge::DGRAD) {
         qh = r / Ge::WU;
         qw = r - qh * Ge::WU;
@@ -471,7 +458,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
         const int oh = g % Ge::OH;
         ok = (g < PACK * Ge::OH) && (ju < Ge::OW) && (n < p.batch);
         pix = ((int64_t)n * Ge::OH + oh) * Ge::OW + ju;
-        n_fwd = n;
       } else {
         const uint32_t q = (uint32_t)tile * 128u + (uint32_t)r;      // < 2^31 (checked by the launcher)
         const uint32_t prow = q / (uint32_t)Ge::WU;
@@ -480,7 +466,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
         const int oh = (int)(prow - n * (uint32_t)Ge::HQ);
         ok = (ju < Ge::OW) && (oh < Ge::OH) && ((int)n < p.batch);
         pix = ((int64_t)n * Ge::OH + oh) * Ge::OW + ju;
-        n_fwd = (int)n;
       }
       // dgrad: the ReLU-mask words of the whole tile row do not depend on the accumulator: fetch them before waiting
       // for the MMAs so that their DRAM latency overlaps the mainloop (they were the top stall of the first version)
@@ -548,7 +533,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
             split_bf16x2(o2, o3, hw[c][2 * j + 1], lw[c][2 * j + 1]);
           }
         }
-        if constexpr (PIPE) pipe_publish(io, note, lane);      // the previous tile's stores (tc2_pipe.cuh: published one tile late)
         if (ok && !(PAACB_DBGV(p.dbg) & 512)) {
 #pragma unroll
           for (int c = 0; c < BN / 32; ++c) {
@@ -561,7 +545,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
             }
           }
         }
-        if constexpr (PIPE) note = pipe_note(io, ok, n_fwd);
         continue;
       }
 #pragma unroll
@@ -625,7 +608,6 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
       tc_fence_before();
       mbar_arrive(&tempty_bar[ab]);
     }
-    if constexpr (PIPE) pipe_publish(io, note, lane);
     if constexpr (Ge::DGRAD) {
       if (p.dbias != nullptr) {
         // column -> channel: PIX == 2 packs two pixels of CH channels into one accumulator row
@@ -642,15 +624,5 @@ __device__ __forceinline__ void convk_body(const ConvKParams& p, const int cta, 
     tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
   }
 }
-
-template <int G>
-__global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __grid_constant__ ConvKParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  convk_body<G, false>(p, (int)blockIdx.x, (int)gridDim.x, smem_raw, PipeIO{});
-}
-
-
-int prepare_conv_fwd_bf16(const paacb_ctx* ctx, int layer, const float* params, void* fwd_ws, int64_t batch, const WsSlice& slice,
-                          ConvKParams* p, int* geo);
 
 }  // namespace paacb

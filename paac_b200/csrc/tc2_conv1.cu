@@ -55,16 +55,15 @@ int launch_pack_conv1_i8(const paacb_ctx* ctx, const float* params, cudaStream_t
   return PAACB_OK;
 }
 
-// fills the kernel parameters (tensor maps of the states and of the int8 digit image, tile count, pointers)
-template <int NC>
-static int prepare_conv1(const paacb_ctx* ctx, const float* params, const uint8_t* states, uint8_t* out_hi, uint8_t* out_lo,
-                         float* out_f32, int64_t batch, Conv1Params* pp) {
+template <int NC, bool F32OUT>
+static int launch_conv1_inst(const paacb_ctx* ctx, const float* params, const uint8_t* states, uint8_t* out_hi, uint8_t* out_lo,
+                             float* out_f32, uint16_t* relu_bits, int64_t batch, cudaStream_t st) {
   const LayerGeom& g = ctx->layer[0];
   if (g.C != 4 || g.stride != 4 || g.R != 8 || g.S != 8 || g.N != NC || g.H != 84 || g.W != 84 || g.OH != kC1_OH)
     return PAACB_EUNSUPPORTED;
   const int64_t plane_rows = batch * kC1_HQ;
   if (plane_rows * kC1_WU >= (1LL << 31) - 256) return PAACB_EUNSUPPORTED;
-  Conv1Params& p = *pp;
+  Conv1Params p;
   memset(&p, 0, sizeof(p));
   // an image row (84 pixels x 4 channels = 336 bytes) is ONE inner box row of 84 32-bit words (box dimensions are limited
   // to 256 elements); plane row q = ih / 4 and row parity rho are separate dimensions (ih = 4 q + rho), parity slowest,
@@ -86,25 +85,6 @@ static int prepare_conv1(const paacb_ctx* ctx, const float* params, const uint8_
   p.out_hi = out_hi;
   p.out_lo = out_lo;
   p.out_f32 = out_f32;
-  return PAACB_OK;
-}
-
-int prepare_conv1_fwd_bf16(const paacb_ctx* ctx, const float* params, const uint8_t* states, void* fwd_ws, int64_t batch,
-                           const WsSlice& slice, Conv1Params* p) {
-  const LayerGeom& g = ctx->layer[0];
-  const Planes out = layer_planes(fwd_ws, g.out_act_off, (int64_t)g.OH * g.OW * g.N, slice);
-  const int rc = (g.N == 16) ? prepare_conv1<16>(ctx, params, states, out.hi, out.lo, nullptr, batch, p)
-                             : prepare_conv1<32>(ctx, params, states, out.hi, out.lo, nullptr, batch, p);
-  if (rc == PAACB_OK) p->relu_bits = reinterpret_cast<uint16_t*>(relu1_bits(fwd_ws, ctx, slice));
-  return rc;
-}
-
-template <int NC, bool F32OUT>
-static int launch_conv1_inst(const paacb_ctx* ctx, const float* params, const uint8_t* states, uint8_t* out_hi, uint8_t* out_lo,
-                             float* out_f32, uint16_t* relu_bits, int64_t batch, cudaStream_t st) {
-  Conv1Params p;
-  const int prc = prepare_conv1<NC>(ctx, params, states, out_hi, out_lo, out_f32, batch, &p);
-  if (prc != PAACB_OK) return prc;
   p.relu_bits = relu_bits;
   constexpr int SMEM = kC1_SMEM_FIXED + C1<NC>::WBYTES;
   static DeviceOnce attr_set;   // kernel attributes are per device: one bit per device index

@@ -1,8 +1,6 @@
-// conv1 forward on the int8 tensor pipe: parameters, geometry and the kernel body (shared by the stand-alone kernel of
-// tc2_conv1.cu and the layer-pipelined forward of tc2_pipe.cu).  Design notes: tc2_conv1.cu.
+// conv1 forward on the int8 tensor pipe: parameters, geometry and the kernel.  Design notes: tc2_conv1.cu.
 #pragma once
 #include "tc2.cuh"
-#include "tc2_pipe.cuh"
 
 namespace paacb {
 
@@ -62,15 +60,13 @@ __host__ __device__ constexpr uint32_t make_idesc_i8(int n) {
   return (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
 }
 
-// SPLIT = warps that share a tile row (each takes NC / SPLIT channels): 2 for the stand-alone Nature kernel (16 epilogue
-// warps hide the TMEM / shared-memory / store latencies of an HBM-bound kernel), 1 in the layer-pipelined forward (8
-// epilogue warps: the CTA is 320 threads like the other layers' roles).  cta / ncta: this CTA's index and count among the
-// CTAs that run this layer.  PIPE: signal the completed samples to the layer below (tc2_pipe.cuh).
-template <int NC, bool F32OUT, int SPLIT, bool PIPE>
-__device__ __forceinline__ void conv1_i8_body(const Conv1Params& p, const int cta, const int ncta, uint8_t* smem_raw, const PipeIO& io) {
+// An epilogue thread owns 16 channels of one tile row: NC / 16 warps share a tile row (Nature: 16 epilogue warps hide the
+// TMEM / shared-memory / barrier / store latencies of an HBM-bound kernel).
+template <int NC, bool F32OUT>
+__global__ void __launch_bounds__(C1<NC>::THREADS, 1) conv1_i8_kernel(const __grid_constant__ Conv1Params p) {
+  const int cta = (int)blockIdx.x, ncta = (int)gridDim.x;   // persistent CTAs: this one's index, their count
   constexpr int kC1_ND = C1<NC>::ND, kC1_WBYTES = C1<NC>::WBYTES;
-  constexpr int HPT = NC / 16 / SPLIT;            // 16-channel groups per thread
-  static_assert(SPLIT == 1 || SPLIT == NC / 16, "one or NC / 16 warps per tile row");
+  extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* ring = smem;
   uint8_t* wsm = smem + kC1_NSLOTS * kC1_SLOT;
@@ -95,7 +91,7 @@ __device__ __forceinline__ void conv1_i8_body(const Conv1Params& p, const int ct
     mbar_init(w_bar, 1);
     for (int s = 0; s < 2; ++s) {
       mbar_init(&tfull_bar[s], 1);
-      mbar_init(&tempty_bar[s], 128 * SPLIT);
+      mbar_init(&tempty_bar[s], 128 * (NC / 16));
     }
     fence_barrier_init();
     tma_prefetch_desc(&p.tmA);
@@ -158,16 +154,14 @@ __device__ __forceinline__ void conv1_i8_body(const Conv1Params& p, const int ct
       if (leader) umma_commit(&tfull_bar[ab]);
       __syncwarp();
     }
-  } else if (warp < 2 + 8 * SPLIT) {
+  } else {
     // =========================== epilogue ===========================
     const int ew = warp & 3;
     const int r = ew * 32 + lane;                   // MMA row = unit r of the tile's 6 x 21 units
     const int grp = ((warp - 2) >> 2) & 1;          // epilogue group = accumulator buffer it drains
-    const int half0 = ((warp - 2) >> 3) * HPT;      // first 16-channel group of this thread: with SPLIT = 2 two warps share a tile
-                                                    // row, which doubles the warps that hide the TMEM / shared-memory / barrier latencies
+    const int cg = (warp - 2) >> 3;                 // this thread's 16-channel group
     const int pr = r / kC1_WU, ju = r - pr * kC1_WU;
     const bool rowok = (r < kC1_TROWS * kC1_WU) && (ju < kC1_OW);
-    PipeNote note = pipe_note_none();
     for (int tl = grp, tile = cta + grp * ncta; tile < p.num_tiles; tile += 2 * ncta, tl += 2) {
       const uint32_t aph = (uint32_t)((tl >> 1) & 1);
       const uint32_t g = (uint32_t)tile * kC1_TROWS + (uint32_t)pr;           // global plane row
@@ -175,44 +169,37 @@ __device__ __forceinline__ void conv1_i8_body(const Conv1Params& p, const int ct
       const bool ok = rowok && ((int)(g - n * (uint32_t)kC1_HQ) < kC1_OH) && ((int)n < p.batch);
       mbar_wait(&tfull_bar[grp], aph);
       tc_fence_after();
-      uint32_t v0[HPT][16], v1[HPT][16], v2[HPT][16];
-#pragma unroll
-      for (int h = 0; h < HPT; ++h) {
-        const uint32_t tcol = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)(grp * 128 + (half0 + h) * 16);
-        tmem_ld16(tcol, v0[h]);
-        tmem_ld16(tcol + (uint32_t)NC, v1[h]);
-        tmem_ld16(tcol + (uint32_t)(2 * NC), v2[h]);
-      }
+      uint32_t v0[16], v1[16], v2[16];
+      const uint32_t tcol = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)(grp * 128 + cg * 16);
+      tmem_ld16(tcol, v0);
+      tmem_ld16(tcol + (uint32_t)NC, v1);
+      tmem_ld16(tcol + (uint32_t)(2 * NC), v2);
       tmem_ld_wait();
       tc_fence_before();
       mbar_arrive(&tempty_bar[grp]);           // the accumulator is in registers: release the buffer before the arithmetic
-      uint32_t hw[HPT][8], lw[HPT][8];
-      float of[F32OUT ? HPT : 1][F32OUT ? 16 : 1];
+      uint32_t hw[8], lw[8];
+      float of[F32OUT ? 16 : 1];
+      const float4* sb4 = reinterpret_cast<const float4*>(s_sb) + cg * 8;
+      if (PAACB_DBGV(p.dbg) & 2) {
 #pragma unroll
-      for (int h = 0; h < HPT; ++h) {
-        const float4* sb4 = reinterpret_cast<const float4*>(s_sb) + (half0 + h) * 8;
-        if (PAACB_DBGV(p.dbg) & 2) {
+        for (int j = 0; j < 8; ++j) { hw[j] = v0[2 * j] ^ v1[2 * j + 1]; lw[j] = v2[2 * j] ^ v0[2 * j + 1]; }
+      } else
 #pragma unroll
-          for (int j = 0; j < 8; ++j) { hw[h][j] = v0[h][2 * j] ^ v1[h][2 * j + 1]; lw[h][j] = v2[h][2 * j] ^ v0[h][2 * j + 1]; }
-        } else
+      for (int j = 0; j < 8; ++j) {
+        const float4 sb = sb4[j];              // (scale, bias) of channels 2j, 2j + 1: one broadcast 16-byte load
+        float o[2];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const float4 sb = sb4[j];              // (scale, bias) of channels 2j, 2j + 1: one broadcast 16-byte load
-          float o[2];
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            // |acc| < 2^22: int -> float exactly on the integer + FMA pipes (the conversion pipe issues at a quarter rate)
-            const float f0 = __uint_as_float(v0[h][2 * j + e] + 0x4B400000u) - 12582912.0f;
-            const float f1 = __uint_as_float(v1[h][2 * j + e] + 0x4B400000u) - 12582912.0f;
-            const float f2 = __uint_as_float(v2[h][2 * j + e] + 0x4B400000u) - 12582912.0f;
-            const float t = fmaf(f2, 1.0f / 4096.0f, fmaf(f1, 1.0f / 64.0f, f0));
-            o[e] = fmaxf(fmaf(t, e ? sb.z : sb.x, e ? sb.w : sb.y), 0.f);
-          }
-          if constexpr (F32OUT) { of[h][2 * j] = o[0]; of[h][2 * j + 1] = o[1]; }
-          else split_bf16x2(o[0], o[1], hw[h][j], lw[h][j]);
+        for (int e = 0; e < 2; ++e) {
+          // |acc| < 2^22: int -> float exactly on the integer + FMA pipes (the conversion pipe issues at a quarter rate)
+          const float f0 = __uint_as_float(v0[2 * j + e] + 0x4B400000u) - 12582912.0f;
+          const float f1 = __uint_as_float(v1[2 * j + e] + 0x4B400000u) - 12582912.0f;
+          const float f2 = __uint_as_float(v2[2 * j + e] + 0x4B400000u) - 12582912.0f;
+          const float t = fmaf(f2, 1.0f / 4096.0f, fmaf(f1, 1.0f / 64.0f, f0));
+          o[e] = fmaxf(fmaf(t, e ? sb.z : sb.x, e ? sb.w : sb.y), 0.f);
         }
+        if constexpr (F32OUT) { of[2 * j] = o[0]; of[2 * j + 1] = o[1]; }
+        else split_bf16x2(o[0], o[1], hw[j], lw[j]);
       }
-      if constexpr (PIPE) pipe_publish(io, note, lane);       // the PREVIOUS tile's stores have had a tile's worth of time to land
       if (ok && !(PAACB_DBGV(p.dbg) & 1)) {                 // 16 channels = one full 32-byte sector per plane
         const uint32_t oh = g - n * (uint32_t)kC1_HQ;
         if constexpr (!F32OUT) {
@@ -222,31 +209,23 @@ __device__ __forceinline__ void conv1_i8_body(const Conv1Params& p, const int ct
             // is <= 0x7f80: no carry between the halves).  Word j's two flags are shifted to bits 15 - j / 31 - j and OR-ed:
             // three instructions per pair of channels in this ALU-bound epilogue; relu1_bit_pos() is the resulting layout.
             const int64_t px = (int64_t)n * (2 * kC1_OH * kC1_OW) + oh * kC1_OW + ju;      // plane 0 of sample n
+            uint32_t acc = 0u;
 #pragma unroll
-            for (int h = 0; h < HPT; ++h) {
-              uint32_t acc = 0u;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) acc |= ((hw[h][j] + 0x7fff7fffu) >> j) & (0x80008000u >> j);
-              const uint32_t bits = ((acc >> 8) & 0xffu) | ((acc >> 16) & 0xff00u);
-              p.relu_bits[px + (half0 + h) * (kC1_OH * kC1_OW)] = (uint16_t)bits;
-            }
+            for (int j = 0; j < 8; ++j) acc |= ((hw[j] + 0x7fff7fffu) >> j) & (0x80008000u >> j);
+            const uint32_t bits = ((acc >> 8) & 0xffu) | ((acc >> 16) & 0xff00u);
+            p.relu_bits[px + cg * (kC1_OH * kC1_OW)] = (uint16_t)bits;
           }
         }
-#pragma unroll
-        for (int h = 0; h < HPT; ++h) {
-          const int64_t oe = (((int64_t)n * kC1_OH + oh) * kC1_OW + ju) * NC + (half0 + h) * 16;      // element index
-          if constexpr (F32OUT) {
-            stg256(p.out_f32 + oe, reinterpret_cast<const uint32_t*>(of[h]));
-            stg256(p.out_f32 + oe + 8, reinterpret_cast<const uint32_t*>(of[h]) + 8);
-          } else {
-            stg256(p.out_hi + oe * 2, hw[h]);
-            stg256(p.out_lo + oe * 2, lw[h]);
-          }
+        const int64_t oe = (((int64_t)n * kC1_OH + oh) * kC1_OW + ju) * NC + cg * 16;      // element index
+        if constexpr (F32OUT) {
+          stg256(p.out_f32 + oe, reinterpret_cast<const uint32_t*>(of));
+          stg256(p.out_f32 + oe + 8, reinterpret_cast<const uint32_t*>(of) + 8);
+        } else {
+          stg256(p.out_hi + oe * 2, hw);
+          stg256(p.out_lo + oe * 2, lw);
         }
       }
-      if constexpr (PIPE) note = pipe_note(io, ok, (int)n);
     }
-    if constexpr (PIPE) pipe_publish(io, note, lane);
   }
 
   tc_fence_before();
@@ -256,15 +235,5 @@ __device__ __forceinline__ void conv1_i8_body(const Conv1Params& p, const int ct
     tmem_dealloc(tmem_base, kC1_TMEM);
   }
 }
-
-template <int NC, bool F32OUT>
-__global__ void __launch_bounds__(C1<NC>::THREADS, 1) conv1_i8_kernel(const __grid_constant__ Conv1Params p) {
-  extern __shared__ uint8_t smem_raw[];
-  conv1_i8_body<NC, F32OUT, NC / 16, false>(p, (int)blockIdx.x, (int)gridDim.x, smem_raw, PipeIO{});
-}
-
-
-int prepare_conv1_fwd_bf16(const paacb_ctx* ctx, const float* params, const uint8_t* states, void* fwd_ws, int64_t batch,
-                           const WsSlice& slice, Conv1Params* p);
 
 }  // namespace paacb

@@ -44,14 +44,13 @@ static int map2d(CUtensorMap* out, const void* base, uint64_t inner, uint64_t ro
   return encode_tmap_bf16(out, base, 2, dims, strides, box, 128);
 }
 
-
-int prepare_fc_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, void* fwd_ws, int64_t batch, const WsSlice& slice,
-                        StreamParams* pp) {
+int launch_fc_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, void* fwd_ws, int64_t batch, const WsSlice& slice,
+                       cudaStream_t st) {
   const LayerGeom& g = ctx->layer[l];
   // K need not be a multiple of the 64-wide K-block (NIPS: 2592 = 40.5 blocks): the TMA engine zero-fills BOTH operands
   // beyond K, so the ragged tail contributes nothing.  Row pitches must be multiples of 16 bytes.
   if (g.K % 8 != 0 || g.N % kFcBN != 0) return PAACB_EUNSUPPORTED;
-  StreamParams& p = *pp;
+  StreamParams p;
   memset(&p, 0, sizeof(p));
   p.dbg = ctx->dbg;
   const Planes x = layer_planes(fwd_ws, g.in_act_off, g.K, slice);
@@ -71,14 +70,6 @@ int prepare_fc_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, void* 
   p.bias = params + g.b_off;
   p.out_hi = y.hi;
   p.out_lo = y.lo;
-  return PAACB_OK;
-}
-
-int launch_fc_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, void* fwd_ws, int64_t batch, const WsSlice& slice,
-                       cudaStream_t st) {
-  StreamParams p;
-  const int rc = prepare_fc_fwd_bf16(ctx, l, params, fwd_ws, batch, slice, &p);
-  if (rc != PAACB_OK) return rc;
   return launch_stream<kFcBN, ST_FWD>(ctx, p, K_FWD0 + l, st);
 }
 

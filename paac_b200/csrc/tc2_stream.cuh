@@ -1,8 +1,7 @@
-// Streaming GEMM of the fully connected layer (forward, data gradient, weight gradient): parameters and the kernel body
-// (shared by the stand-alone kernels of tc2_stream.cu and the layer-pipelined forward of tc2_pipe.cu).  Design: tc2_stream.cu.
+// Streaming GEMM of the fully connected layer (forward, data gradient, weight gradient): parameters and the kernel.
+// Design: tc2_stream.cu.
 #pragma once
 #include "tc2.cuh"
-#include "tc2_pipe.cuh"
 
 namespace paacb {
 
@@ -56,14 +55,13 @@ __device__ __forceinline__ float warp_transpose_sum32(float (&v)[32], int lane) 
   return v[0];
 }
 
-// cta / ncta: this CTA's index and count among the CTAs that run this GEMM (warps beyond kStreamThreads / 32 idle).  PIPE
-// (forward): before the first K-block of a unit the TMA producer waits until the 128 samples of its m-tile are complete in
-// the layer above (one counter per 128 samples, tc2_pipe.cuh).
-template <int BN, int MODE, bool PIPE>
-__device__ __forceinline__ void stream_gemm_body(const StreamParams& p, const int cta, const int ncta, uint8_t* smem_raw, const PipeIO& io) {
+template <int BN, int MODE>
+__global__ void __launch_bounds__(kStreamThreads, 1) stream_gemm_kernel(const __grid_constant__ StreamParams p) {
+  const int cta = (int)blockIdx.x, ncta = (int)gridDim.x;   // persistent CTAs: this one's index, their count
   using Cfg = StreamCfg<BN, MODE>;
   constexpr int STAGES = Cfg::STAGES;
   constexpr bool MN = Cfg::MN;
+  extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + STAGES * Cfg::STAGE_BYTES);
   uint64_t* full_bar = bars;
@@ -119,10 +117,6 @@ __device__ __forceinline__ void stream_gemm_body(const StreamParams& p, const in
         int split, mt, nt, kb0, kb1;
         decode(u, split, mt, nt);
         kb_range(split, kb0, kb1);
-        if constexpr (PIPE) {
-          const int rows = p.M - mt * 128 < 128 ? p.M - mt * 128 : 128;        // samples of this m-tile
-          pipe_wait_one(io, mt, io.up_target * (uint32_t)rows);
-        }
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(&empty_bar[stage], phase ^ 1u);
           if (PAACB_DBGV(p.dbg) & 2048) { mbar_arrive(&full_bar[stage]); if (++stage == STAGES) { stage = 0; phase ^= 1u; } continue; }
@@ -190,7 +184,7 @@ __device__ __forceinline__ void stream_gemm_body(const StreamParams& p, const in
       if (leader) umma_commit(&tfull_bar[ab]);
       __syncwarp();
     }
-  } else if (warp < kStreamThreads / 32) {
+  } else {
     // =========================== epilogue ===========================
     const int ew = warp & 3;
     const int r = ew * 32 + lane;
@@ -317,15 +311,5 @@ __device__ __forceinline__ void stream_gemm_body(const StreamParams& p, const in
     tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
   }
 }
-
-template <int BN, int MODE>
-__global__ void __launch_bounds__(kStreamThreads, 1) stream_gemm_kernel(const __grid_constant__ StreamParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  stream_gemm_body<BN, MODE, false>(p, (int)blockIdx.x, (int)gridDim.x, smem_raw, PipeIO{});
-}
-
-
-int prepare_fc_fwd_bf16(const paacb_ctx* ctx, int layer, const float* params, void* fwd_ws, int64_t batch, const WsSlice& slice,
-                        StreamParams* p);
 
 }  // namespace paacb

@@ -109,18 +109,6 @@ class Network(object):
         _lib.check(self._lib.paacb_set_math(self.ctx, mode), 'paacb_set_math')
         self.math = str(math).lower()
 
-    def set_forward_pipeline(self, enable=True, ctas=(0, 0, 0)):
-        """bf16x3, opt-in experiment (measured slower than one launch per layer, DESIGN 3.3; off by default): run conv1 ...
-        hidden fc of a forward as ONE layer-pipelined persistent kernel; ``ctas`` = CTAs given to conv1, conv2, conv3 (0: keep the library's split; the fc layer takes the other SMs).
-        Both schedules produce the same bits (tests/test_gpu_pipe.py)."""
-        _lib.check(self._lib.paacb_set_forward_pipeline(self.ctx, 1 if enable else 0, int(ctas[0]), int(ctas[1]), int(ctas[2])),
-                   'paacb_set_forward_pipeline')
-
-    def forward_pipeline_errors(self):
-        out = C.c_uint32(0)
-        _lib.check(self._lib.paacb_forward_pipeline_errors(self.ctx, C.byref(out)), 'paacb_forward_pipeline_errors')
-        return int(out.value)
-
     def initialize(self, seed=None):
         """'torch' init of networks.py:24-46,63-81: U(-d, d), d = 1/sqrt(fan_in), weights AND biases."""
         rng = np.random.RandomState(seed)

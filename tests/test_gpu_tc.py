@@ -218,6 +218,62 @@ def test_cached_weight_images_follow_the_parameters():
     assert not np.array_equal(v1, v2)
 
 
+@pytest.mark.parametrize('arch', ['NATURE', 'NIPS'])
+def test_forward_bits_do_not_depend_on_slices_or_streams(arch):
+    """The bf16x3 forward of a batch leaves the same bits in the activation workspace, pi and v whether it is issued whole or
+    as ragged slices of one workspace (paacb_policy_forward_at), also after new parameters, and when the forwards of two
+    batches alternate on two streams."""
+    A = 6
+    net = G.make_net(arch, A, seed=13, math='bf16x3')
+    gen = torch.Generator(device='cuda'); gen.manual_seed(6)
+    states = torch.randint(0, 256, (600, 84, 84, 4), dtype=torch.uint8, device='cuda', generator=gen)
+
+    def run(s):
+        b = s.shape[0]
+        pi = torch.full((b, A), -1.0, device='cuda'); v = torch.full((b,), -1.0, device='cuda')
+        ws = torch.zeros((net.workspace_floats(b),), device='cuda')
+        net.forward(s, pi, v, ws)
+        torch.cuda.synchronize()
+        return ws.view(torch.int32).clone(), pi, v
+
+    def sliced():
+        pi = torch.zeros((600, A), device='cuda'); v = torch.zeros((600,), device='cuda')
+        ws = torch.zeros((net.workspace_floats(600),), device='cuda')
+        for lo, hi in ((0, 250), (250, 251), (251, 600)):
+            net.forward(states[lo:hi], pi[lo:hi], v[lo:hi], ws, ws_capacity=600, ws_first=lo)
+        torch.cuda.synchronize()
+        return ws.view(torch.int32).clone(), pi, v
+
+    whole = run(states)
+    for a, b in zip(whole, sliced()):
+        assert torch.equal(a, b)
+    # new parameters: the cached operand images are refreshed
+    net.set_params(net.get_params() * np.float32(0.5))
+    whole_new, sliced_new = run(states), sliced()
+    for a, b in zip(whole_new, sliced_new):
+        assert torch.equal(a, b)
+    assert not torch.equal(sliced_new[2], whole[2])
+
+    sa = torch.randint(0, 256, (2000, 84, 84, 4), dtype=torch.uint8, device='cuda', generator=gen)
+    sb = torch.randint(0, 256, (1500, 84, 84, 4), dtype=torch.uint8, device='cuda', generator=gen)
+    ra, rb = run(sa), run(sb)
+    outs = []
+    streams = [torch.cuda.Stream(), torch.cuda.Stream()]
+    for s in (sa, sb):
+        b = s.shape[0]
+        pi = torch.zeros((b, A), device='cuda'); v = torch.zeros((b,), device='cuda')
+        ws = torch.zeros((net.workspace_floats(b),), device='cuda')
+        outs.append((ws, pi, v))
+    torch.cuda.synchronize()
+    for rep in range(3):
+        for st, s, (ws, pi, v) in zip(streams, (sa, sb), outs):
+            with torch.cuda.stream(st):
+                net.forward(s, pi, v, ws)
+    torch.cuda.synchronize()
+    for ref, (ws, pi, v) in zip((ra, rb), outs):
+        assert torch.equal(ref[0], ws.view(torch.int32)) and torch.equal(ref[1], pi) and torch.equal(ref[2], v)
+
+
 def test_sliced_bootstrap_equals_whole_batch():
     """RolloutEngine.bootstrap(lo, hi) per environment slice (what the end-to-end loop issues as each slice's last frames
     arrive) leaves the same V(s_T), loss and update as the whole-batch bootstrap inside update()."""

@@ -109,15 +109,6 @@ int paacb_observe_u8(const paacb_ctx* ctx, const uint8_t* d_frames, int pairs_pe
                      const float* d_over_in, float* d_rewards_out, float* d_over_out, int over_is_reset,
                      paacb_stream stream);
 
-/* SURVEY 8(f) rank 1 (frame-dedup rollout storage), prototype pair used for the measured A/B in DESIGN.md section 6:
- * K1 at its contract traffic -- the new 84x84 plane only, into slot `slot` of a planar ring uint8 [n_envs, ring_slots, 84, 84]
- * (ring_slots >= 4; a rollout needs t_max + 3) -- and the gather that rebuilds the NHWC stack [n_envs, 84, 84, 4] from the
- * four newest slots (channel 3 = newest_slot, oldest first), which is what conv1's operand layout still needs. */
-int paacb_preprocess_planar_u8(const paacb_ctx* ctx, const uint8_t* d_frames, int pairs_per_env, uint8_t* d_ring,
-                               int ring_slots, int slot, int64_t n_envs, paacb_stream stream);
-int paacb_stack_from_planes(const paacb_ctx* ctx, const uint8_t* d_ring, int ring_slots, int newest_slot, uint8_t* d_next,
-                            int64_t n_envs, paacb_stream stream);
-
 /* ---- K2-K6: forward (+ sampling).  Replaces session.run([output_layer_v, output_layer_pi])
  * and __sample_policy_action (paac.py:18-45).
  *   d_params   float [P]               d_states uint8 [b,84,84,4]

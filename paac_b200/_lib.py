@@ -42,8 +42,6 @@ PROTOTYPES = {
                                      _vp, _vp, _vp, _vp, _vp, _vp]),
     'paacb_backward': (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     'paacb_clip_rmsprop': (_i, [_vp, _vp, _vp, _vp, _vp, _f, _f, _f, _f, _f, _f, _i, _vp, _vp, _vp]),
-    'paacb_preprocess_planar_u8': (_i, [_vp, _vp, _i, _vp, _i, _i, _i64, _vp]),
-    'paacb_stack_from_planes': (_i, [_vp, _vp, _i, _i, _vp, _i64, _vp]),
     'paacb_observe_u8': (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, _vp]),
     'paacb_policy_forward_sample': (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _vp, C.c_uint64, _i64, _vp, _vp, _vp]),
     'paacb_rng_advance': (_i, [_vp, _vp, C.c_uint64, _vp]),

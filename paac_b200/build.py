@@ -21,10 +21,6 @@ NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
 ARCH_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a']
 CFLAGS = ['-O3', '-std=c++17', '-lineinfo', '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr',
           '-Xptxas', '-v' if os.environ.get('PAACB_PTXAS_V') else '-warn-spills']
-if os.environ.get('PAACB_ABLATIONS'):          # measurement build: keeps the PAACB_DBG ablation switches in the kernels
-    CFLAGS.append('-DPAACB_ABLATIONS')
-    OBJ_DIR = os.path.join(ROOT, 'build', 'paacb_abl')
-    LIB = os.path.join(HERE, 'libpaacb_abl.so')
 
 
 def sources():

@@ -126,22 +126,8 @@ int paacb_create(paacb_ctx** out, int arch, int num_actions, int device) {
   c->arch = arch; c->num_actions = num_actions; c->device = device; c->math = PAACB_MATH_FP32;
   c->num_sms = prop.multiProcessorCount;
   c->opt_fused_blocks = -1;
-  {
-    const char* knob = getenv("PAACB_DBG");
-    c->dbg = (knob != nullptr) ? atoi(knob) : 0;
-    const char* ap = getenv("PAACB_ALWAYS_PACK");
-    c->always_pack = (ap != nullptr) ? atoi(ap) : 0;
-    const char* tp = getenv("PAACB_OPT_TWO_PASS");
-    c->opt_two_pass = (tp != nullptr) ? atoi(tp) : 0;
-    const char* hg = getenv("PAACB_K1_HOST_GRID");      // tuning knob for tools/experiments/pcie_probe.py
-    c->k1_host_grid = (hg != nullptr && atoi(hg) > 0) ? atoi(hg) : 96;
-    const char* kp = getenv("PAACB_K1_PIPE");
-    c->k1_pipe = (kp != nullptr) ? atoi(kp) : 2;
-    const char* kg = getenv("PAACB_K1_PIPE_HOST_GRID");
-    c->k1_pipe_host_grid = (kg != nullptr && atoi(kg) > 0) ? atoi(kg) : 32;
-    const char* kh = getenv("PAACB_K1_HINTS");
-    c->k1_hints = (kh != nullptr) ? atoi(kh) : 3;
-  }
+  const char* tp = getenv("PAACB_OPT_TWO_PASS");
+  c->opt_two_pass = (tp != nullptr) ? atoi(tp) : 0;
   int h = PAACB_OBS, w = PAACB_OBS, ch = PAACB_STACK;
   int64_t poff = 0, aoff = 0;
   if (arch == PAACB_ARCH_NIPS) {                       // networks.py:145-149
@@ -195,14 +181,6 @@ int paacb_create(paacb_ctx** out, int arch, int num_actions, int device) {
       c->opt_counter = nullptr;          // falls back to the two-launch optimizer
     }
     cudaSetDevice(cur);
-  }
-  {
-    const char* c3 = getenv("PAACB_CONV3_PACKED");
-    c->conv3_packed = (c3 != nullptr) ? atoi(c3) : 1;
-    const char* rk = getenv("PAACB_SM_RESERVE_KERNELS");
-    c->sm_reserve_kernels = (rk != nullptr) ? atoi(rk) : 3;
-    const char* e = getenv("PAACB_PDL");
-    c->pdl_on = (e == nullptr) ? 1 : atoi(e);
   }
   *out = c;
   return PAACB_OK;
@@ -386,7 +364,7 @@ static int pack_forward_images(const paacb_ctx* ctx, const float* d_params, cuda
   return PAACB_OK;
 }
 static int ensure_forward_images(const paacb_ctx* ctx, const float* d_params, cudaStream_t st) {
-  if (ctx->fwd_img_valid && ctx->fwd_img_src == d_params && !ctx->always_pack) return PAACB_OK;
+  if (ctx->fwd_img_valid && ctx->fwd_img_src == d_params) return PAACB_OK;
   const int rc = pack_forward_images(ctx, d_params, st);
   if (rc == PAACB_OK) {
     ctx->fwd_img_valid = 1;
@@ -461,33 +439,13 @@ int paacb_observe_u8(const paacb_ctx* ctx, const uint8_t* d_frames, int pairs_pe
   return preprocess_impl(ctx, d_frames, pairs_per_env, d_reset, d_prev, d_next, n_envs, sc, stream);
 }
 
-int paacb_preprocess_planar_u8(const paacb_ctx* ctx, const uint8_t* d_frames, int pairs_per_env, uint8_t* d_ring,
-                               int ring_slots, int slot, int64_t n_envs, paacb_stream stream) {
-  PAACB_CHECK_ARG(ctx && d_frames && d_ring, "NULL argument");
-  PAACB_CHECK_DEVICE(ctx);
-  PAACB_CHECK_ARG(pairs_per_env >= 1 && ring_slots >= PAACB_STACK && slot >= 0 && slot < ring_slots, "pairs / ring slot out of range");
-  PAACB_CHECK_ARG(n_envs >= 0 && n_envs < (1LL << 31), "n_envs out of range");
-  PAACB_CHECK_ARG(((uintptr_t)d_frames & 15) == 0 && ((uintptr_t)d_ring & 15) == 0, "buffers must be 16-byte aligned");
-  return launch_preprocess_planar(ctx, d_frames, pairs_per_env, d_ring, ring_slots, slot, n_envs, (cudaStream_t)stream);
-}
-
-int paacb_stack_from_planes(const paacb_ctx* ctx, const uint8_t* d_ring, int ring_slots, int newest_slot, uint8_t* d_next,
-                            int64_t n_envs, paacb_stream stream) {
-  PAACB_CHECK_ARG(ctx && d_ring && d_next, "NULL argument");
-  PAACB_CHECK_DEVICE(ctx);
-  PAACB_CHECK_ARG(ring_slots >= PAACB_STACK && newest_slot >= 0 && newest_slot < ring_slots, "ring slot out of range");
-  PAACB_CHECK_ARG(n_envs >= 0 && n_envs < (1LL << 31), "n_envs out of range");
-  PAACB_CHECK_ARG(((uintptr_t)d_next & 15) == 0 && ((uintptr_t)d_ring & 15) == 0, "buffers must be 16-byte aligned");
-  return launch_stack_from_planes(ctx, d_ring, ring_slots, newest_slot, d_next, n_envs, (cudaStream_t)stream);
-}
-
 static int run_layer_fwd(const paacb_ctx* ctx, int l, const float* d_params, const uint8_t* d_states, int64_t batch,
                          float* ws, const WsSlice& slice, cudaStream_t st) {
   const LayerGeom& g = ctx->layer[l];
   const void* x = (l == 0) ? (const void*)d_states
                            : (const void*)(ws + g.in_act_off * slice.cap + slice.first * (int64_t)g.H * g.W * g.C);
   float* y = ws + g.out_act_off * slice.cap + slice.first * (int64_t)g.OH * g.OW * g.N;
-  if (ctx->math != PAACB_MATH_FP32 && l == 0 && g.N == 16 && ctx->wq_i8 != nullptr && !(PAACB_DBGV(ctx->dbg) & (1 << 17))) {
+  if (ctx->math != PAACB_MATH_FP32 && l == 0 && g.N == 16 && ctx->wq_i8 != nullptr) {
     // NIPS conv1: uint8 pixels x int8 weight digits (tc2_conv1.cu; the digit image is part of the cached forward images)
     const int rc = launch_conv1_fwd_i8_f32(ctx, d_params, d_states, y, batch, st);
     if (rc != PAACB_EUNSUPPORTED) return rc;

@@ -10,15 +10,6 @@
 #error "paacb is written for sm_100a (B200) only"
 #endif
 
-// Ablation switches (PAACB_DBG bit mask: stages of a kernel switched off for timing experiments, tools/ablation_sweep.py)
-// exist only in builds made with PAACB_ABLATIONS=1 (python -m paac_b200.build); in the product build they compile to 0 and
-// the branches vanish from the kernels.
-#ifdef PAACB_ABLATIONS
-#define PAACB_DBGV(x) (x)
-#else
-#define PAACB_DBGV(x) 0
-#endif
-
 namespace paacb {
 
 // One conv / fc layer viewed as an implicit GEMM: Y[M, N] = im2col(X)[M, K] * W[K, N].
@@ -120,22 +111,12 @@ struct paacb_ctx {
   unsigned int* opt_counter;
   mutable int opt_fused_blocks;
   int opt_two_pass;             // PAACB_OPT_TWO_PASS=1: the two-launch optimizer (sumsq + update)
-  int always_pack;              // PAACB_ALWAYS_PACK=1: re-derive the images on every forward (debug)
-  // K1: memory type of the frame buffers seen so far (address >> 21 -> host?) and the narrow grid of the zero-copy launch
+  // K1: memory type of the frame buffers seen so far (address >> 21 -> host?)
   static constexpr int kK1Cache = 8;
   mutable int k1_cache_n;
   mutable uintptr_t k1_cache_key[kK1Cache];
   mutable int k1_cache_host[kK1Cache];
-  int k1_host_grid;             // PAACB_K1_HOST_GRID (default 96)
-  int k1_pipe;                  // PAACB_K1_PIPE (default 2): 0 = CTA-per-environment kernel only, 1 = device-resident frames go through the persistent
-                                // copy pipeline, 2 = pinned host frames too (on k1_pipe_host_grid CTAs: PCIe needs few loads in flight)
-  int k1_pipe_host_grid;        // PAACB_K1_PIPE_HOST_GRID (default 32)
-  int k1_hints;                 // PAACB_K1_HINTS (default 3): bit 0 = inputs read evict-first, bit 1 = new stack written evict-last
-  int conv3_packed;             // PAACB_CONV3_PACKED (default 1): conv3 forward with two whole samples per tile (tc2_conv.cuh: Geo<G_FWD3P>)
-  int pdl_on;                   // PAACB_PDL (default 1): programmatic dependent launch between the kernels of one forward / backward
-  int sm_reserve_kernels;       // PAACB_SM_RESERVE_KERNELS (default 3): how many of the conv weight-gradient kernels, in launch order, leave them
   int sm_reserve;               // paacb_set_sm_reserve: SMs the persistent conv weight-gradient kernels leave free (multi-GPU)
-  int dbg;                      // PAACB_DBG: ablation switches of the tcgen05 kernels for timing experiments (0 in production)
 };
 
 namespace paacb {
@@ -152,9 +133,9 @@ void set_error(const char* fmt, ...);
 
 void prof_drain(const paacb_ctx* ctx);
 
-// kernel<<<grid, block, smem, st>>>(args...), optionally with the programmatic-stream-serialization attribute (tc_ptx.cuh)
+// kernel<<<grid, block, smem, st>>>(args...) with the programmatic-stream-serialization attribute (tc_ptx.cuh)
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_kernel(void (*kern)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t st, bool pdl,
+inline cudaError_t launch_kernel(void (*kern)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t st,
                                  Args&&... args) {
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -166,7 +147,7 @@ inline cudaError_t launch_kernel(void (*kern)(KArgs...), unsigned grid, unsigned
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 // bracket a kernel launch: PAACB_LAUNCH_BEGIN(ctx, kid, st); kernel<<<...>>>(...); PAACB_LAUNCH_END(ctx, kid, st);
@@ -195,11 +176,6 @@ inline cudaError_t launch_kernel(void (*kern)(KArgs...), unsigned grid, unsigned
 // ---- launchers implemented in the .cu files (all asynchronous on `st`) --------------------------
 int launch_preprocess(const paacb_ctx* ctx, const uint8_t* frames, int pairs, const uint8_t* reset,
                       const uint8_t* prev, uint8_t* next, int64_t n, const StepScalars& sc, cudaStream_t st);
-
-int launch_preprocess_planar(const paacb_ctx* ctx, const uint8_t* frames, int pairs, uint8_t* ring, int ring_slots, int slot,
-                             int64_t n, cudaStream_t st);
-int launch_stack_from_planes(const paacb_ctx* ctx, const uint8_t* ring, int ring_slots, int newest_slot, uint8_t* next, int64_t n,
-                             cudaStream_t st);
 
 // SIMT fp32 implicit GEMMs (gemm_simt.cu)
 int launch_conv_fwd_simt(const paacb_ctx* ctx, const LayerGeom& g, const void* x, const float* w, const float* bias,

@@ -390,10 +390,10 @@ int launch_heads_fwd(const paacb_ctx* ctx, const float* h, const uint16_t* h_hi,
   if (h == nullptr && (F == 512 || F == 256)) {
     PAACB_LAUNCH_BEGIN(ctx, K_HEADS_FWD, st);
     if (F == 512)
-      launch_kernel(heads_fwd_split_kernel<512>, (unsigned)blocks, kHeadWarps * 32, smem, st, ctx->pdl_on != 0, h_hi, h_lo, wa, ba, wc, bc,
+      launch_kernel(heads_fwd_split_kernel<512>, (unsigned)blocks, kHeadWarps * 32, smem, st, h_hi, h_lo, wa, ba, wc, bc,
                     batch, A, pi, v, smp, actions, onehot);
     else
-      launch_kernel(heads_fwd_split_kernel<256>, (unsigned)blocks, kHeadWarps * 32, smem, st, ctx->pdl_on != 0, h_hi, h_lo, wa, ba, wc, bc,
+      launch_kernel(heads_fwd_split_kernel<256>, (unsigned)blocks, kHeadWarps * 32, smem, st, h_hi, h_lo, wa, ba, wc, bc,
                     batch, A, pi, v, smp, actions, onehot);
     PAACB_LAUNCH_END(ctx, K_HEADS_FWD, st);
     return PAACB_OK;

@@ -119,8 +119,6 @@ struct TcParams {
   int Hq, Wq, I;          // dgrad: class grid and taps per row
   float in_scale;
   int relu;
-  int dbg;                // ablation switches for timing experiments (PAACB_DBG): 1 skip B copy, 2 skip tcgen05.st, 4 skip cp.async,
-                          // 8 skip the MMAs, 16 skip the epilogue stores.  Results are wrong when non-zero.
 };
 
 constexpr int kSmemBudget = 224 * 1024;      // B stages + cp.async staging (the per-SM maximum is 227 KB incl. static)
@@ -286,7 +284,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
           }
           const uint8_t* src = ok ? xb + (base_j[j] + tab) * ESZ + my_chunk * 16 : xb;   // !ok: 0 bytes read, zero fill
           const int row = j * RPI + my_row0;
-          if (!(PAACB_DBGV(p.dbg) & 4)) cp_async16(dst0 + (uint32_t)(row * Cfg::ROWB) + (((uint32_t)my_chunk ^ swz_of(row)) << 4), src, ok ? 16u : 0u);
+          cp_async16(dst0 + (uint32_t)(row * Cfg::ROWB) + (((uint32_t)my_chunk ^ swz_of(row)) << 4), src, ok ? 16u : 0u);
         }
       }
       ld_kb += NG * KSUB;
@@ -324,14 +322,10 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
           mbar_wait(&empty_bar[pstage], pphase ^ 1u);
           if (wq4 == 0 && elect_one_sync()) {
             uint8_t* b_hi = smem + (size_t)pstage * Cfg::STAGE_BYTES;
-            if (PAACB_DBGV(p.dbg) & 1) {
-              mbar_arrive(&full_bar[pstage]);
-            } else {
-              mbar_arrive_expect_tx(&full_bar[pstage], Cfg::STAGE_BYTES);
-              bulk_g2s(b_hi, p.b_hi + (int64_t)img * (BN * 32), KSUB * Cfg::B_BYTES, &full_bar[pstage]);
-              if constexpr (SPLIT)
-                bulk_g2s(b_hi + KSUB * Cfg::B_BYTES, p.b_lo + (int64_t)img * (BN * 32), KSUB * Cfg::B_BYTES, &full_bar[pstage]);
-            }
+            mbar_arrive_expect_tx(&full_bar[pstage], Cfg::STAGE_BYTES);
+            bulk_g2s(b_hi, p.b_hi + (int64_t)img * (BN * 32), KSUB * Cfg::B_BYTES, &full_bar[pstage]);
+            if constexpr (SPLIT)
+              bulk_g2s(b_hi + KSUB * Cfg::B_BYTES, p.b_lo + (int64_t)img * (BN * 32), KSUB * Cfg::B_BYTES, &full_bar[pstage]);
           }
           // this thread's row of the A operand goes straight into tensor memory: lane = row, 32 columns per K-block
 #pragma unroll
@@ -347,7 +341,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
                 hi[c * 4 + 2] = __float_as_uint(u8_to_f32(wds[c], 2));
                 hi[c * 4 + 3] = __float_as_uint(u8_to_f32(wds[c], 3));
               }
-              if (!(PAACB_DBGV(p.dbg) & 2)) tmem_st32(taddr, hi);
+              tmem_st32(taddr, hi);
             } else {
               // TF32X3: hi = a with the 13 low mantissa bits cleared (1 LOP), lo = a - hi exactly (1 FADD); the tensor
               // core reads only the tf32 bits of lo, an error of 2^-21 |a|.  Plain TF32 rounds to nearest (2 integer ops).
@@ -358,7 +352,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
                 hi[c * 4 + 2] = Cfg::A_LO ? (b[sb][c].z & 0xFFFFE000u) : tf32_rna_bits(b[sb][c].z);
                 hi[c * 4 + 3] = Cfg::A_LO ? (b[sb][c].w & 0xFFFFE000u) : tf32_rna_bits(b[sb][c].w);
               }
-              if (!(PAACB_DBGV(p.dbg) & 2)) tmem_st32(taddr, hi);
+              tmem_st32(taddr, hi);
               if constexpr (Cfg::A_LO) {
                 uint32_t lo[32];
 #pragma unroll
@@ -368,7 +362,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
                   lo[c * 4 + 2] = __float_as_uint(__uint_as_float(b[sb][c].z) - __uint_as_float(hi[c * 4 + 2]));
                   lo[c * 4 + 3] = __float_as_uint(__uint_as_float(b[sb][c].w) - __uint_as_float(hi[c * 4 + 3]));
                 }
-                if (!(PAACB_DBGV(p.dbg) & 2)) tmem_st32(taddr + 32u, lo);
+                tmem_st32(taddr + 32u, lo);
               }
             }
           }
@@ -402,28 +396,26 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
           tc_fence_after();
           const uint32_t b_st = smem_u32(smem + (size_t)stage * Cfg::STAGE_BYTES);
           if (leader) {
-          if (!(PAACB_DBGV(p.dbg) & 8)) {
 #pragma unroll
-          for (int sb = 0; sb < KSUB; ++sb) {
-            const uint32_t b_hi = b_st + (uint32_t)(sb * Cfg::B_BYTES), b_lo = b_hi + (uint32_t)(KSUB * Cfg::B_BYTES);
+            for (int sb = 0; sb < KSUB; ++sb) {
+              const uint32_t b_hi = b_st + (uint32_t)(sb * Cfg::B_BYTES), b_lo = b_hi + (uint32_t)(KSUB * Cfg::B_BYTES);
 #pragma unroll
-            for (int ks = 0; ks < 4; ++ks) {   // K = 8 tf32 per instruction: 32 bytes of smem (B) / 8 TMEM columns (A)
-              const uint32_t ko = (uint32_t)ks * 32u;
-              uint32_t accum = (kb > 0 || sb > 0 || ks > 0) ? 1u : 0u;
-              const uint32_t a_hi = tmem_base + kAcol0 + (uint32_t)(stage * Cfg::SCOLS + sb * Cfg::ACOLS) + (uint32_t)ks * 8u;
-              if constexpr (SPLIT) {
-                if constexpr (Cfg::A_LO) {
-                  umma_tf32_ts(d_tmem, a_hi + 32u, make_sw128_desc(b_hi + ko), idesc, accum);
+              for (int ks = 0; ks < 4; ++ks) {   // K = 8 tf32 per instruction: 32 bytes of smem (B) / 8 TMEM columns (A)
+                const uint32_t ko = (uint32_t)ks * 32u;
+                uint32_t accum = (kb > 0 || sb > 0 || ks > 0) ? 1u : 0u;
+                const uint32_t a_hi = tmem_base + kAcol0 + (uint32_t)(stage * Cfg::SCOLS + sb * Cfg::ACOLS) + (uint32_t)ks * 8u;
+                if constexpr (SPLIT) {
+                  if constexpr (Cfg::A_LO) {
+                    umma_tf32_ts(d_tmem, a_hi + 32u, make_sw128_desc(b_hi + ko), idesc, accum);
+                    accum = 1u;
+                  }
+                  umma_tf32_ts(d_tmem, a_hi, make_sw128_desc(b_lo + ko), idesc, accum);
                   accum = 1u;
                 }
-                umma_tf32_ts(d_tmem, a_hi, make_sw128_desc(b_lo + ko), idesc, accum);
-                accum = 1u;
+                umma_tf32_ts(d_tmem, a_hi, make_sw128_desc(b_hi + ko), idesc, accum);
               }
-              umma_tf32_ts(d_tmem, a_hi, make_sw128_desc(b_hi + ko), idesc, accum);
             }
-          }
-          }
-          umma_commit(&empty_bar[stage]);      // stage reusable once these MMAs retire
+            umma_commit(&empty_bar[stage]);      // stage reusable once these MMAs retire
           }
           __syncwarp();
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
@@ -479,7 +471,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) igemm_tc_kernel(const TcParams 
           tmem_ld32(taddr + (uint32_t)c0, v);
           tmem_ld_wait();
         }
-        if (ok && !(PAACB_DBGV(p.dbg) & 16)) {
+        if (ok) {
           float* dst = p.y + out_base + c0;
           if constexpr (MODE == TC_DGRAD) {
             const float* xa = (p.xact != nullptr) ? p.xact + out_base + c0 : nullptr;
@@ -551,7 +543,7 @@ static int launch_tc_inst(const paacb_ctx* ctx, const TcParams& p, int slot, int
   // K-blocks per pipeline stage: 4 for the uint8 layer (32-byte rows: small stages are all handshake); the fp32
   // layers measured faster with single-K-block stages (deeper TMEM / smem pipelines, fewer live registers)
   constexpr int KS = (MODE == TC_FWD_U8) ? 4 : 1;
-  if (KS > 1 && p.kblocks % KS == 0 && !(PAACB_DBGV(ctx->dbg) & 32)) {
+  if (KS > 1 && p.kblocks % KS == 0) {
     return split3 ? launch_tc_inst2<BN, MODE, true, KS>(ctx, p, slot, st) : launch_tc_inst2<BN, MODE, false, KS>(ctx, p, slot, st);
   }
   return split3 ? launch_tc_inst2<BN, MODE, true, 1>(ctx, p, slot, st) : launch_tc_inst2<BN, MODE, false, 1>(ctx, p, slot, st);
@@ -610,7 +602,6 @@ int launch_conv_fwd_tc(const paacb_ctx* ctx, const LayerGeom& g, const void* x, 
   p.kblocks = g.K / 32;
   p.in_scale = g.in_u8 ? 0.003921568859368563f : 1.0f;
   p.relu = 1;
-  p.dbg = ctx->dbg;
   const int slot = K_FWD0 + g.index;
   if (g.in_u8) {
     if (bn == 16) return launch_tc_inst<16, TC_FWD_U8>(ctx, p, slot, split3, st);
@@ -652,7 +643,6 @@ int launch_conv_dgrad_tc(const paacb_ctx* ctx, const LayerGeom& g, const float* 
   p.classes = s * s;
   p.kblocks = J * I * g.N / 32;
   p.in_scale = 1.0f;
-  p.dbg = ctx->dbg;
   const int slot = K_DGRAD0 + g.index;
   if (bn == 16) return launch_tc_inst<16, TC_DGRAD>(ctx, p, slot, split3, st);
   if (bn == 32) return launch_tc_inst<32, TC_DGRAD>(ctx, p, slot, split3, st);

@@ -110,15 +110,15 @@ preprocess_u8_kernel(const uint8_t* __restrict__ frames, int pairs, const uint8_
 //                      selected rows are each a uniform 800-byte pitch that also runs across frames (33,600 = 42 x 800),
 //                      so ONE rank-3 tensor map per parity {160 B, 42 rows, frames} with a box of {160, 42, 2} lands the
 //                      42 rows of both frames of a pair.  (First version: 168 bulk copies of 160 B per environment --
-//                      2.4x SLOWER than the kernel above, ~60 cycles of TMA issue per copy; measured, tools/gpu_round2_t.sh.)
+//                      2.4x SLOWER than the kernel above, ~60 cycles of TMA issue per copy; profiles/r02_k1_pipeline_ab.txt.)
 //   warps 2-9          wait `full`, turn the stage's stack into the next stack IN PLACE ((prev >> 8) | max(f0, f1) << 24 per
 //                      pixel word; column table and row offsets live in registers for the whole kernel),
 //                      fence.proxy.async, arrive on `done`
 //   warp 1 (storer)    wait `done`, ONE 28,224-byte bulk store shared -> global, wait until the engine has read the stage,
 //                      arrive on `empty`
 // No thread touches global memory on the fast path (resets -- rare, 4 pairs per environment -- are gathered straight from
-// global memory by the consumer warps into the same stage).  L2 policy (PAACB_K1_HINTS): bit 0 = the frame rows and the
-// old stack are read evict-first (never used again), bit 1 = the new stack is written evict-last.
+// global memory by the consumer warps into the same stage).  L2 policy: the frame rows and the old stack are read
+// evict-first (never used again), the new stack is written evict-last.
 // The launcher falls back to the kernel above when the row table is not the affine pattern.
 // ------------------------------------------------------------------------------------------------------------------
 constexpr int kK1Stages = 4;
@@ -139,16 +139,19 @@ struct K1PipeParams {
   const uint8_t* prev;
   uint8_t* next;
   int64_t n_envs;
-  int pairs, hints;
+  int pairs;
   StepScalars sc;
   ResizeTables tabs;
 };
 
-__device__ __forceinline__ uint64_t l2_policy(int kind) {   // 0 normal, 1 evict-first, 2 evict-last
+__device__ __forceinline__ uint64_t l2_evict_first() {
   uint64_t pol;
-  if (kind == 1) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  else if (kind == 2) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  else asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
+  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+  return pol;
+}
+__device__ __forceinline__ uint64_t l2_evict_last() {
+  uint64_t pol;
+  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
 __device__ __forceinline__ void bulk_g2s_hint(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar, uint64_t pol) {
@@ -191,7 +194,7 @@ __global__ void __launch_bounds__(kK1PipeThreads, 1) preprocess_u8_pipe_kernel(c
     if (lane == 0) {
       tma_prefetch_desc(&p.tm_even);
       tma_prefetch_desc(&p.tm_odd);
-      const uint64_t pol = l2_policy((p.hints & 1) ? 1 : 0);
+      const uint64_t pol = l2_evict_first();
       int k = 0;
       for (int64_t env = blockIdx.x; env < p.n_envs; env += gridDim.x, ++k) {
         const int s = k % kK1Stages;
@@ -208,7 +211,7 @@ __global__ void __launch_bounds__(kK1PipeThreads, 1) preprocess_u8_pipe_kernel(c
   } else if (warp == 1) {
     // ---- storer ----
     if (lane == 0) {
-      const uint64_t pol = l2_policy((p.hints & 2) ? 2 : 0);
+      const uint64_t pol = l2_evict_last();
       int k = 0;
       for (int64_t env = blockIdx.x; env < p.n_envs; env += gridDim.x, ++k) {
         const int s = k % kK1Stages;
@@ -297,110 +300,20 @@ __global__ void __launch_bounds__(kK1PipeThreads, 1) preprocess_u8_pipe_kernel(c
   }
 }
 
-// ------------------------------------------------------------------------------------------------------------------
-// SURVEY 8(f) rank 1, frame-dedup rollout storage -- the measured half of the A/B (DESIGN 6).  K1 at its CONTRACT traffic:
-// the two frames' 84 selected rows in (26,880 B), ONE new 84 x 84 plane out (7,056 B) into a planar ring
-// uint8 [n_envs, ring_slots, 84, 84]; a rollout of T steps then needs T + 3 planes per environment instead of T stacked
-// [84, 84, 4] copies (paac.py:92,112 stores every frame four times).  stack_from_planes_kernel rebuilds the NHWC stack the
-// conv1 kernels consume from four ring slots (oldest first) -- the cost a planar ring adds back for as long as conv1's
-// int8 implicit GEMM needs its 16-byte (4 pixels x 4 frames) units.  tools/microbench_cfg5.py times both against K1.
-// ------------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kThreads)
-preprocess_planar_u8_kernel(const uint8_t* __restrict__ frames, int pairs, uint8_t* __restrict__ ring, int ring_slots, int slot,
-                            ResizeTables tabs, int64_t n_envs) {
-  __shared__ __align__(16) uint8_t plane[PAACB_OBS * PAACB_FRAME_W];
-  __shared__ int s_row[PAACB_OBS];
-  __shared__ int s_col[PAACB_OBS];
-  const int tid = threadIdx.x;
-  if (tid < PAACB_OBS) {
-    s_row[tid] = tabs.row[tid] * PAACB_FRAME_W;
-    s_col[tid] = tabs.col[tid];
-  }
-  for (int64_t env = blockIdx.x; env < n_envs; env += gridDim.x) {
-    const uint8_t* f0 = frames + (env * pairs * 2) * (int64_t)kFrameBytes;
-    const uint8_t* f1 = f0 + kFrameBytes;
-    __syncthreads();
-    for (int i = tid; i < PAACB_OBS * kRowVec; i += kThreads) {
-      const int y = i / kRowVec, c = i - y * kRowVec;
-      const int src = s_row[y] + c * 16;
-      const uint4 a = __ldg(reinterpret_cast<const uint4*>(f0 + src));
-      const uint4 b = __ldg(reinterpret_cast<const uint4*>(f1 + src));
-      uint4 m;
-      m.x = __vmaxu4(a.x, b.x); m.y = __vmaxu4(a.y, b.y); m.z = __vmaxu4(a.z, b.z); m.w = __vmaxu4(a.w, b.w);
-      *reinterpret_cast<uint4*>(plane + y * PAACB_FRAME_W + c * 16) = m;
-    }
-    __syncthreads();
-    // 84 x 84 bytes = 441 uint4 per plane: 16 output pixels per thread-iteration
-    uint4* out = reinterpret_cast<uint4*>(ring + (env * ring_slots + slot) * (int64_t)(PAACB_OBS * PAACB_OBS));
-    for (int i = tid; i < PAACB_OBS * PAACB_OBS / 16; i += kThreads) {
-      uint32_t w[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        uint32_t v = 0;
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const int px = i * 16 + j * 4 + e;
-          const int y = px / PAACB_OBS, x = px - y * PAACB_OBS;
-          v |= (uint32_t)plane[y * PAACB_FRAME_W + s_col[x]] << (8 * e);
-        }
-        w[j] = v;
-      }
-      out[i] = make_uint4(w[0], w[1], w[2], w[3]);
-    }
-  }
-}
-
-__global__ void __launch_bounds__(kThreads)
-stack_from_planes_kernel(const uint8_t* __restrict__ ring, int ring_slots, int newest_slot, uint8_t* __restrict__ next, int64_t n_envs) {
-  const int tid = threadIdx.x;
-  for (int64_t env = blockIdx.x; env < n_envs; env += gridDim.x) {
-    const uint8_t* base = ring + env * ring_slots * (int64_t)(PAACB_OBS * PAACB_OBS);
-    const uint32_t* pl[PAACB_STACK];
-#pragma unroll
-    for (int c = 0; c < PAACB_STACK; ++c)        // channel c = the frame 3 - c steps back, oldest first
-      pl[c] = reinterpret_cast<const uint32_t*>(base + ((newest_slot - 3 + c + 4 * ring_slots) % ring_slots) * (int64_t)(PAACB_OBS * PAACB_OBS));
-    uint4* out = reinterpret_cast<uint4*>(next + env * (int64_t)(kStateVec * 16));
-    for (int i = tid; i < kStateVec; i += kThreads) {       // 4 pixels = one 32-bit word of each plane -> one uint4 of the stack
-      const uint32_t a = __ldg(pl[0] + i), b = __ldg(pl[1] + i), c = __ldg(pl[2] + i), d = __ldg(pl[3] + i);
-      // [a0 b0 a1 b1], [c0 d0 c1 d1] ... then pixel words [a b c d] (channel 0 = oldest frame in the low byte)
-      const uint32_t ab01 = __byte_perm(a, b, 0x5140), cd01 = __byte_perm(c, d, 0x5140);
-      const uint32_t ab23 = __byte_perm(a, b, 0x7362), cd23 = __byte_perm(c, d, 0x7362);
-      uint4 o;
-      o.x = __byte_perm(ab01, cd01, 0x5410);
-      o.y = __byte_perm(ab01, cd01, 0x7632);
-      o.z = __byte_perm(ab23, cd23, 0x5410);
-      o.w = __byte_perm(ab23, cd23, 0x7632);
-      out[i] = o;
-    }
-  }
-}
-
-int launch_preprocess_planar(const paacb_ctx* ctx, const uint8_t* frames, int pairs, uint8_t* ring, int ring_slots, int slot,
-                             int64_t n, cudaStream_t st) {
-  if (n == 0) return PAACB_OK;
-  PAACB_LAUNCH_BEGIN(ctx, K_PREPROCESS, st);
-  preprocess_planar_u8_kernel<<<(unsigned)n, kThreads, 0, st>>>(frames, pairs, ring, ring_slots, slot, ctx->tabs, n);
-  PAACB_LAUNCH_END(ctx, K_PREPROCESS, st);
-  return PAACB_OK;
-}
-
-int launch_stack_from_planes(const paacb_ctx* ctx, const uint8_t* ring, int ring_slots, int newest_slot, uint8_t* next, int64_t n,
-                             cudaStream_t st) {
-  if (n == 0) return PAACB_OK;
-  PAACB_LAUNCH_BEGIN(ctx, K_PREPROCESS, st);
-  stack_from_planes_kernel<<<(unsigned)n, kThreads, 0, st>>>(ring, ring_slots, newest_slot, next, n);
-  PAACB_LAUNCH_END(ctx, K_PREPROCESS, st);
-  return PAACB_OK;
-}
+// Launch shapes of K1 on frames in pinned, mapped host memory (read zero-copy, PCIe-bound: few loads in flight are enough,
+// and the other SMs stay free for the tensor-core kernels of the next environment slice).  The pipeline's TMA row reads
+// cross PCIe at 43.1 GB/s against 42.0 for the threads' 16-byte loads, and on 32 CTAs instead of 96 the end-to-end cycle
+// went 16.37 -> 15.8-15.95 ms (profiles/r02_k1_pipeline_ab.txt).
+constexpr int kK1PipeHostGrid = 32;      // CTAs of the copy pipeline
+constexpr int kK1HostGrid = 96;          // grid-stride grid of the CTA-per-environment kernel
 
 int launch_preprocess(const paacb_ctx* ctx, const uint8_t* frames, int pairs, const uint8_t* reset,
                       const uint8_t* prev, uint8_t* next, int64_t n, const StepScalars& sc, cudaStream_t st) {
   if (n == 0) return PAACB_OK;
   // Two kernels.  More than one environment per SM: the persistent TMA copy pipeline (above) -- one CTA per SM for device-resident
-  // frames (HBM-bound), PAACB_K1_PIPE_HOST_GRID CTAs for frames in pinned, mapped HOST memory (the runners' buffers, read
-  // zero-copy: PCIe-bound, few loads in flight are enough, and the other SMs stay free for the tensor-core kernels of the next
-  // environment slice).  Small batches, or a row table that is not the two-pitch pattern: the CTA-per-environment kernel
-  // (host frames: as a narrow grid-stride grid, PAACB_K1_HOST_GRID).
+  // frames (HBM-bound), kK1PipeHostGrid CTAs for frames in pinned, mapped HOST memory (the runners' buffers).  Small batches,
+  // or a row table that is not the two-pitch pattern: the CTA-per-environment kernel (host frames: as a narrow grid-stride
+  // grid of kK1HostGrid CTAs).
   unsigned grid = (unsigned)n;
   // is the frame buffer host memory?  The answer is cached per 2 MB-aligned address range the caller has used (a runner's
   // buffer is registered once and then read every step: no driver query on the hot path)
@@ -417,19 +330,12 @@ int launch_preprocess(const paacb_ctx* ctx, const uint8_t* frames, int pairs, co
     ctx->k1_cache_key[slot] = key;
     ctx->k1_cache_host[slot] = is_host;
   }
-  if (is_host) {
-    unsigned narrow = (unsigned)ctx->k1_host_grid;
-    if (n > narrow) grid = narrow;
-  }
+  if (is_host && n > kK1HostGrid) grid = kK1HostGrid;
   bool affine = true;       // row(2k) = row(0) + 5k, row(2k + 1) = row(1) + 5k: what the two row-parity tensor maps can express
   for (int y = 0; y < PAACB_OBS; ++y) affine = affine && ((int)ctx->tabs.row[y] == (int)ctx->tabs.row[y & 1] + 5 * (y >> 1));
   // (a CTA of the pipeline needs at least two environments to overlap anything: batches up to one environment per SM -- the
   // reference's default 32 -- keep the CTA-per-environment kernel)
-  // PAACB_K1_PIPE=2 (default): pinned host frames go through the pipeline too, on PAACB_K1_PIPE_HOST_GRID CTAs -- the TMA engine's
-  // row reads cross PCIe at 43.1 GB/s against 42.0 for the threads' 16-byte loads (tools/experiments/pcie_probe.py), 32 SMs are
-  // held instead of 96, and the end-to-end cycle went 16.37 -> 15.8-15.95 ms (tools/gpu_round2_y.sh)
-  const bool pipe_host = is_host && ctx->k1_pipe == 2;
-  if ((!is_host || pipe_host) && ctx->k1_pipe && affine && n > (int64_t)ctx->num_sms &&
+  if (affine && n > (int64_t)ctx->num_sms &&
       (((uintptr_t)frames | (uintptr_t)prev | (uintptr_t)next) & 15) == 0 && n * pairs * 2 < (1LL << 31)) {
     static DeviceOnce attr_once;
     if (!attr_once.done(ctx->device)) {
@@ -449,8 +355,8 @@ int launch_preprocess(const paacb_ctx* ctx, const uint8_t* frames, int pairs, co
     if (rc == PAACB_OK) rc = encode_tmap(&p.tm_odd, frames + (int)ctx->tabs.row[1] * PAACB_FRAME_W, 1, 3, dims, strides, box, 0);
     if (rc != PAACB_OK) return rc;
     p.frames = frames; p.reset = reset; p.prev = prev; p.next = next;
-    p.n_envs = n; p.pairs = pairs; p.hints = ctx->k1_hints; p.sc = sc; p.tabs = ctx->tabs;
-    const unsigned pgrid = (unsigned)((pipe_host && ctx->k1_pipe_host_grid < ctx->num_sms) ? ctx->k1_pipe_host_grid : ctx->num_sms);
+    p.n_envs = n; p.pairs = pairs; p.sc = sc; p.tabs = ctx->tabs;
+    const unsigned pgrid = (unsigned)((is_host && kK1PipeHostGrid < ctx->num_sms) ? kK1PipeHostGrid : ctx->num_sms);
     PAACB_LAUNCH_BEGIN(ctx, K_PREPROCESS, st);
     preprocess_u8_pipe_kernel<<<pgrid, kK1PipeThreads, kK1PipeSmem, st>>>(p);
     PAACB_LAUNCH_END(ctx, K_PREPROCESS, st);

@@ -192,7 +192,7 @@ static int launch_convk(const paacb_ctx* ctx, const ConvKParams& p, int slot, cu
   }
   const unsigned grid = (unsigned)(p.num_tiles < ctx->num_sms ? p.num_tiles : ctx->num_sms);
   PAACB_LAUNCH_BEGIN(ctx, slot, st);
-  launch_kernel(convk_kernel<G>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, st, ctx->pdl_on != 0, p);
+  launch_kernel(convk_kernel<G>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, st, p);
   PAACB_LAUNCH_END(ctx, slot, st);
   return PAACB_OK;
 }
@@ -213,7 +213,6 @@ int launch_conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const
   ConvKParams p;
   memset(&p, 0, sizeof(p));
   p.batch = (int)batch;
-  p.dbg = ctx->dbg;
   p.bias = params + g.b_off;
   p.in_scale = g.in_u8 ? 0.003921568859368563f : 1.0f;
   const Planes out = layer_planes(fwd_ws, g.out_act_off, (int64_t)g.OH * g.OW * g.N, slice);
@@ -254,7 +253,7 @@ int launch_conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const
   // (each case leaves its do-while with `break` when the layer's geometry is not the one it was written for)
   if (l == 1) do PAACB_FWD_CASE(G_FWD2) while (0);
   if (l == 1) do PAACB_FWD_CASE(G_FWD2N) while (0);
-  if (l == 2 && ctx->conv3_packed) do {
+  if (l == 2) do {
     // conv3, two whole samples per tile (Geo<G_FWD3P>): the source planes as (channels, x, y, sample); one box = the 7 input
     // rows kh .. kh + 6 of two samples; a box that runs past the last sample is zero-filled
     using Ge = Geo<G_FWD3P>;
@@ -272,7 +271,6 @@ int launch_conv_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, const
     p.num_tiles = (int)((batch + GeoPack<G_FWD3P>::SAMPLES - 1) / GeoPack<G_FWD3P>::SAMPLES);
     return launch_convk<G_FWD3P>(ctx, p, K_FWD0 + l, st);
   } while (0);
-  if (l == 2) do PAACB_FWD_CASE(G_FWD3) while (0);
 #undef PAACB_FWD_CASE
   return PAACB_EUNSUPPORTED;
 }
@@ -285,7 +283,6 @@ int launch_conv_dgrad_bf16(const paacb_ctx* ctx, int l, const void* fwd_ws, void
   ConvKParams p;
   memset(&p, 0, sizeof(p));
   p.batch = (int)batch;
-  p.dbg = ctx->dbg;
   p.num_tiles = (int)batch;
   const Planes dz = layer_planes(bwd_ws, g.out_act_off, (int64_t)g.OH * g.OW * g.N, batch);
   const Planes dx = layer_planes(bwd_ws, gp.out_act_off, (int64_t)g.H * g.W * g.C, batch);
@@ -316,8 +313,7 @@ int launch_conv_dgrad_bf16(const paacb_ctx* ctx, int l, const void* fwd_ws, void
       const uint64_t od[4] = {(uint64_t)2 * g.C, (uint64_t)g.W / 2, 2u, (uint64_t)batch * (g.H / 2)};              \
       const uint64_t os[3] = {(uint64_t)2 * g.C * 2, (uint64_t)g.W * g.C * 2, (uint64_t)2 * g.W * g.C * 2};        \
       const uint32_t ob[4] = {(uint32_t)(2 * g.C), (uint32_t)(g.W / 2), 1u, (uint32_t)(g.H / 2)};                  \
-      rc = encode_tmap_bf16(&p.tmOut[0], dx.hi, 4, od, os, ob, 128);                                               \
-      if (rc == PAACB_OK) rc = encode_tmap_bf16(&p.tmOut[1], dx.lo, 4, od, os, ob, 128);                           \
+      rc = encode_tmap_bf16(&p.tmOut, dx.hi, 4, od, os, ob, 128);                                                  \
     }                                                                                                              \
     if (rc != PAACB_OK) return rc;                                                                                 \
     return launch_convk<GE>(ctx, p, K_DGRAD0 + l, st);                                                             \

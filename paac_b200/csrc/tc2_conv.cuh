@@ -8,7 +8,7 @@ namespace paacb {
 // ------------------------------------------------------------------------------------------------
 // geometry of the five patch-resident GEMMs of the Nature network
 // ------------------------------------------------------------------------------------------------
-enum { G_FWD2 = 1, G_FWD3 = 2, G_DG3 = 3, G_DG2 = 4,        // Nature; conv1 forward has its own int8 kernel (tc2_conv1.cu)
+enum { G_FWD2 = 1, G_DG3 = 3, G_DG2 = 4,                    // Nature; conv1 forward has its own int8 kernel (tc2_conv1.cu)
        G_FWD2N = 5, G_DG2N = 6,                             // NIPS conv2 (networks.py:146): 64-byte units, SWIZZLE_64B
        G_FWD3P = 7 };                                       // conv3 forward, two whole samples per tile (below)
 
@@ -25,23 +25,14 @@ struct Geo<G_FWD2> {
   __host__ __device__ static constexpr int aoff(int t) { return ((t / 8) * 10 + ((t / 4) % 2)) * 128 + (t % 4) * 32; }
   __host__ __device__ static constexpr int jw(int part, int t) { return ((part + 2 * (t / 8)) * 2 + ((t / 4) % 2)) * 4 + (t % 4); }
 };
-// conv3 forward: [b,9,9,64] 3x3 stride 1 -> [b,7,7,64].  Unit = 1 pixel x 64 channels = 128 B.
-template <>
-struct Geo<G_FWD3> {
-  static constexpr bool DGRAD = false, A_LO = true, STAGED = false, MASK_BITS = false;
-  static constexpr int UB = 128, SWZ = SWZ_128B, PARTS = 1, WU = 9, HQ = 9, BOX_ROWS = 18, SLOT = 21504, NSLOTS = 3;
-  static constexpr int NACC = 1, BN = 64, KS = 36, KB = 9, OH = 7, OW = 7;
-  static constexpr int CH = 64, PIX = 1;
-  __host__ __device__ static constexpr int aoff(int t) { return (((t / 4) / 3) * 9 + ((t / 4) % 3)) * 128 + (t % 4) * 32; }
-  __host__ __device__ static constexpr int jw(int, int t) { return t; }
-};
-// conv3 forward, PACKED (round 2): the geometry above enumerates the 9 x 9 INPUT grid, of which 7 x 7 positions are outputs
-// (60 % of the MMA rows).  A row group of an MMA operand is 8 consecutive 128-byte units and the groups lie at a uniform
-// stride (the descriptor's SBO, any multiple of 16 bytes: probe A_k128_sbo1152) -- so group g = output row (sample g / 7,
-// oh = g % 7), its 8 units = ow 0..7 (7 outputs), stride 9 units, over a patch copy that holds ONLY the 7 input rows
-// kh .. kh + 6 of each sample: the TMA box {64 ch, 9, 7 rows from kh, 2 samples} lands exactly that, densely.  One copy per
-// filter row kh (PARTS = 3; the 2nd and 3rd are L2 hits), tap (kh, kw) = copy kh at a byte offset of kw units.  A tile = two
-// whole samples = 14 of 16 groups x 7 of 8 units: 77 % of the MMA rows, 0.5 instead of 0.63 tiles per sample.
+// conv3 forward: [b,9,9,64] 3x3 stride 1 -> [b,7,7,64].  Unit = 1 pixel x 64 channels = 128 B.  PACKED: enumerating the 9 x 9
+// INPUT grid, as conv2's forward does, would make only 7 x 7 positions outputs (60 % of the MMA rows).  A row group of an MMA
+// operand is 8 consecutive 128-byte units and the groups lie at a uniform stride (the descriptor's SBO, any multiple of 16
+// bytes: probe A_k128_sbo1152) -- so group g = output row (sample g / 7, oh = g % 7), its 8 units = ow 0..7 (7 outputs), stride
+// 9 units, over a patch copy that holds ONLY the 7 input rows kh .. kh + 6 of each sample: the TMA box {64 ch, 9, 7 rows from
+// kh, 2 samples} lands exactly that, densely.  One copy per filter row kh (PARTS = 3; the 2nd and 3rd are L2 hits), tap (kh, kw)
+// = copy kh at a byte offset of kw units.  A tile = two whole samples = 14 of 16 groups x 7 of 8 units: 77 % of the MMA rows,
+// 0.5 instead of 0.63 tiles per sample.
 template <>
 struct Geo<G_FWD3P> {
   static constexpr bool DGRAD = false, A_LO = true, STAGED = false, MASK_BITS = false;
@@ -114,7 +105,7 @@ struct Geo<G_DG2N> {
 struct ConvKParams {
   CUtensorMap tmA[2];      // source planes (hi, lo); forward: dims (unit, units/row, row parity, plane rows); dgrad: (C, OW, OH, b)
   CUtensorMap tmW[2];      // packed weights (hi, lo): dims (K, rows)
-  CUtensorMap tmOut[2];    // staged epilogue: output planes (hi, lo) as (2 px x C, W/2, row parity, b * H/2)
+  CUtensorMap tmOut;       // staged epilogue: output hi plane as (2 px x C, W/2, row parity, b * H/2)
   int num_tiles;
   int batch;
   const float* bias;       // forward
@@ -123,7 +114,6 @@ struct ConvKParams {
   uint8_t* out_lo;
   const uint8_t* mask_hi;  // dgrad: hi plane of the activation whose ReLU is differentiated (same shape as the output)
   const uint32_t* mask_bits;   // conv2's data gradient: the same mask as bit planes, uint16 [b][2][XH * XW] (tc2.cuh: relu1_bits)
-  int dbg;                 // PAACB_DBG ablations (timing experiments only): 256 no A_lo MMAs, 512 no stores, 1024 no patch loads, 4096 conv2 dgrad: lo plane through the staging tile, 8192 conv2 dgrad: both planes by direct stores (measured: no gain once the staging tile is gone)
   float* dbias;            // dgrad: += column sums of the output (the bias gradient of the layer that produced that activation)
 };
 
@@ -139,7 +129,7 @@ struct ConvKCfg {
   static constexpr int W_BYTES = Ge::KB * KB_BYTES;
   static constexpr int BOX_BYTES = Ge::UB * Ge::WU * Ge::BOX_ROWS;
   static constexpr int STG_TILE = 13 * 1024;                                // 100 rows x 128 B, 1024-byte aligned
-  static constexpr int STG_BYTES = Ge::STAGED ? 2 * STG_TILE : 0;            // one tile per output-row parity: hi plane, then lo plane
+  static constexpr int STG_BYTES = Ge::STAGED ? 2 * STG_TILE : 0;            // one tile of the hi plane per output-row parity
   static constexpr int NBARS = 2 * Ge::NSLOTS + 1 + 4 + 1;
   static constexpr int SMEM_BYTES = RING_BYTES + W_BYTES + STG_BYTES + 1024 /* alignment slack */ + NBARS * 8 + 16 + 256 /* forward: bias row */;
   static constexpr int TMEM_COLS = 4 * NT;                                  // two accumulator buffers of 2 * NT columns
@@ -232,11 +222,11 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
       uint32_t phase = 0;
       for (int tile = cta; tile < p.num_tiles; tile += ncta) {
         // (requesting the boxes of the tile after next into L2 with cp.async.bulk.prefetch.tensor was measured: 3 % slower; the
-        // packed conv3 geometry with the NEXT tile's two samples prefetched: 0.603 -> 0.617 ms per step, tools/gpu_round2_x.sh;
+        // packed conv3 geometry with the NEXT tile's two samples prefetched: 0.603 -> 0.617 ms per step;
         // prefetch.global.L2 of the tile after next by the idle epilogue threads, one per 128-byte line: conv2 0.76-0.79 -> 0.79-0.83,
-        // conv3 unchanged, tools/gpu_round2_z.sh -- these kernels do not wait for first-touch DRAM latency)
-        // slot order: (part, piece) with the piece fastest; PACKED: piece slowest, so that the MMAs run in the same order as in
-        // the input-grid geometry (all taps of A_hi, then all taps of A_lo) and the accumulators hold the same bits
+        // conv3 unchanged -- these kernels do not wait for first-touch DRAM latency)
+        // slot order: (part, piece) with the piece fastest; PACKED: piece slowest (all taps of A_hi, then all taps of A_lo: the
+        // MMA order of the input-grid conv3 forward it replaced, so that the accumulators hold the same bits)
         constexpr int NPIECE = Ge::A_LO ? 2 : 1;
 #pragma unroll 1
         for (int it = 0; it < Ge::PARTS * NPIECE; ++it) {
@@ -244,7 +234,6 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
           const int piece = PACK > 0 ? it / Ge::PARTS : it % NPIECE;
           {
             mbar_wait(&empty_bar[slot], phase ^ 1u);
-            if (PAACB_DBGV(p.dbg) & 1024) { mbar_arrive(&full_bar[slot]); if (++slot == NSLOTS) { slot = 0; phase ^= 1u; } continue; }
             mbar_arrive_expect_tx(&full_bar[slot], Cfg::BOX_BYTES);
             uint8_t* dst = ring + slot * Ge::SLOT;
             if constexpr (Ge::DGRAD) {
@@ -297,7 +286,7 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
               const int jw = Ge::jw(part, t);
               const uint64_t bd = desc_with_addr(bdesc0, w_a + (uint32_t)((jw / 4) * Cfg::KB_BYTES + (jw % 4) * 32));
               if (piece == 0) umma_bf16(d0, ad, bd, idesc_full, (part | t) ? 1u : 0u);    // A_hi * [W_hi | W_lo]
-              else if (!(PAACB_DBGV(p.dbg) & 256)) umma_bf16(d0, ad, bd, idesc_half, 1u);              // A_lo * W_hi
+              else umma_bf16(d0, ad, bd, idesc_half, 1u);                                             // A_lo * W_hi
             }
             umma_commit(&empty_bar[slot]);
           }
@@ -335,13 +324,13 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
         return make_uint2(__ldg(reinterpret_cast<const uint32_t*>(b)), __ldg(reinterpret_cast<const uint32_t*>(b + Ge::XH * Ge::XW)));
       };
       uint2 mb_next = make_uint2(0u, 0u);
-      if (ok && cta < p.num_tiles && !(PAACB_DBGV(p.dbg) & 16384)) mb_next = load_bits(cta);
+      if (ok && cta < p.num_tiles) mb_next = load_bits(cta);
       int tl = 0;
       for (int tile = cta; tile < p.num_tiles; tile += ncta, ++tl) {
         const int ab = tl & 1;
         const uint32_t aph = (uint32_t)((tl >> 1) & 1);
         const uint2 mb = mb_next;
-        if (ok && tile + ncta < p.num_tiles && !(PAACB_DBGV(p.dbg) & 16384)) mb_next = load_bits(tile + ncta);
+        if (ok && tile + ncta < p.num_tiles) mb_next = load_bits(tile + ncta);
         mbar_wait(&tfull_bar[ab], aph);
         tc_fence_after();
         float o[2][32];
@@ -360,67 +349,39 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
         }
         tc_fence_before();
         mbar_arrive(&tempty_bar[ab]);                                       // accumulator drained: the MMAs of tile tl + 2 may start
-        // This group's 100 x 128 B staging tile carries the hi plane, then the lo plane (shared memory is needed for a
+        // This group's 100 x 128 B staging tile carries the hi plane only (the rest of shared memory is needed for a
         // 4-deep patch ring: with 2 slots the kernel was bound by the TMA round trip).  io = the group's first thread.
         uint8_t* tile_p = stg + ph * Cfg::STG_TILE;
         const uint32_t t_row = stg_a + (uint32_t)(ph * Cfg::STG_TILE) + srow * 128u;
         uint32_t lw[2][16];
-        const bool direct_hi = (PAACB_DBGV(p.dbg) & 8192) != 0;                         // experiment: no staging at all
-        if (!direct_hi) {
-          if (io) tma_store_wait_read();                                    // previous tile's hi plane has been read out
-          named_bar_sync(1 + ph, 128);
-        }
+        if (io) tma_store_wait_read();                                      // previous tile's hi plane has been read out
+        named_bar_sync(1 + ph, 128);
 #pragma unroll
         for (int pw = 0; pw < 2; ++pw) {
           uint32_t hw[16];
 #pragma unroll
           for (int j = 0; j < 16; ++j) split_bf16x2(o[pw][2 * j], o[pw][2 * j + 1], hw[j], lw[pw][j]);
           if (ok) {
-            if (direct_hi) {
-              uint8_t* dh = p.out_hi + ((((int64_t)tile * Ge::XH + Ge::S * qh + ph) * Ge::XW + Ge::S * qw) * BN) * 2;
 #pragma unroll
-              for (int c = 0; c < 2; ++c) stg256(dh + pw * 64 + c * 32, &hw[8 * c]);
-            } else {
-#pragma unroll
-              for (int c = 0; c < 4; ++c)                                   // 16-byte chunk pw * 4 + c of the row, swizzled
-                sts128(t_row + ((((uint32_t)(pw * 4 + c)) ^ (srow & 7u)) << 4), make_uint4(hw[4 * c], hw[4 * c + 1], hw[4 * c + 2], hw[4 * c + 3]));
-            }
+            for (int c = 0; c < 4; ++c)                                     // 16-byte chunk pw * 4 + c of the row, swizzled
+              sts128(t_row + ((((uint32_t)(pw * 4 + c)) ^ (srow & 7u)) << 4), make_uint4(hw[4 * c], hw[4 * c + 1], hw[4 * c + 2], hw[4 * c + 3]));
           }
         }
-        if (!direct_hi) {
-          fence_proxy_async();                                              // staging writes -> visible to the TMA engine
-          named_bar_sync(1 + ph, 128);
-          if (io) {
-            tma_store_4d(&p.tmOut[0], tile_p, 0, 0, ph, tile * Ge::OH);
-            tma_store_commit();
-          }
+        fence_proxy_async();                                                // staging writes -> visible to the TMA engine
+        named_bar_sync(1 + ph, 128);
+        if (io) {
+          tma_store_4d(&p.tmOut, tile_p, 0, 0, ph, tile * Ge::OH);
+          tma_store_commit();
         }
         // bias gradient: channel = lane for both classes: add the classes first, ONE transposed warp reduction per tile
         // (this kernel has no registers left for per-thread column sums; the shuffles overlap the TMA engine reading the tile)
 #pragma unroll
         for (int j = 0; j < 32; ++j) o[0][j] += o[1][j];
         bsum += warp_transpose_sum(o[0], lane);
-        if (PAACB_DBGV(p.dbg) & 4096) {
-          // (first staged version, kept for A/B timing: the lo plane follows the hi plane through the same staging tile --
-          // two more barriers and a second wait for the TMA engine per tile)
-          if (io) tma_store_wait_read();
-          named_bar_sync(1 + ph, 128);
-          if (ok) {
-#pragma unroll
-            for (int pw = 0; pw < 2; ++pw)
-#pragma unroll
-              for (int c = 0; c < 4; ++c)
-                sts128(t_row + ((((uint32_t)(pw * 4 + c)) ^ (srow & 7u)) << 4), make_uint4(lw[pw][4 * c], lw[pw][4 * c + 1], lw[pw][4 * c + 2], lw[pw][4 * c + 3]));
-          }
-          fence_proxy_async();
-          named_bar_sync(1 + ph, 128);
-          if (io) {
-            tma_store_4d(&p.tmOut[1], tile_p, 0, 0, ph, tile * Ge::OH);
-            tma_store_commit();
-          }
-        } else if (ok) {
+        if (ok) {
           // lo plane: this thread's two pixels are one 128-byte row of the plane -- four 256-bit stores straight from
-          // registers while the TMA engine drains the hi tile (there is no shared memory for a second staging tile)
+          // registers while the TMA engine drains the hi tile (there is no shared memory for a second staging tile; sending
+          // the lo plane through the same tile after the hi plane costs two more barriers and a second wait per tile)
           uint8_t* dl = p.out_lo + ((((int64_t)tile * Ge::XH + Ge::S * qh + ph) * Ge::XW + Ge::S * qw) * BN) * 2;
 #pragma unroll
           for (int pw = 0; pw < 2; ++pw)
@@ -477,7 +438,7 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
         for (int acc = 0; acc < NACC; ++acc) {
           const int ih = Ge::S * qh + acc, iw = Ge::S * qw;
           mbits[acc] = 0u;
-          if (ok && !(PAACB_DBGV(p.dbg) & 16384))      // plane 0 of sample `tile`: pixels iw, iw + 1 are one aligned 32-bit word
+          if (ok)      // plane 0 of sample `tile`: pixels iw, iw + 1 are one aligned 32-bit word
             mbits[acc] = __ldg(reinterpret_cast<const uint32_t*>(reinterpret_cast<const uint16_t*>(p.mask_bits) +
                                                                  (int64_t)tile * (2 * Ge::XH * Ge::XW) + ih * Ge::XW + iw));
         }
@@ -493,7 +454,7 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
           for (int c = 0; c < BN / 32; ++c) {
 #pragma unroll
             for (int j = 0; j < 4; ++j) mk[acc][c][j] = make_uint4(0u, 0u, 0u, 0u);
-            if (ok && !(PAACB_DBGV(p.dbg) & 16384)) {
+            if (ok) {
               ldg256(p.mask_hi + (ob + c * 32) * 2, mk[acc][c][0], mk[acc][c][1]);
               ldg256(p.mask_hi + (ob + c * 32) * 2 + 32, mk[acc][c][2], mk[acc][c][3]);
             }
@@ -533,7 +494,7 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
             split_bf16x2(o2, o3, hw[c][2 * j + 1], lw[c][2 * j + 1]);
           }
         }
-        if (ok && !(PAACB_DBGV(p.dbg) & 512)) {
+        if (ok) {
 #pragma unroll
           for (int c = 0; c < BN / 32; ++c) {
             uint8_t* dh = p.out_hi + (pix * BN + c * 32) * 2;
@@ -587,7 +548,7 @@ __global__ void __launch_bounds__(ConvKCfg<G>::THREADS, 1) convk_kernel(const __
               o[2 * j + 1] = (ok && a1 != 0u && a1 < 0x8000u) ? __uint_as_float(v[2 * j + 1]) : 0.f;
             }
           }
-          if (ok && !(PAACB_DBGV(p.dbg) & 512)) {
+          if (ok) {
             uint32_t hw[16], lw[16];
 #pragma unroll
             for (int j = 0; j < 16; ++j) split_bf16x2(o[2 * j], o[2 * j + 1], hw[j], lw[j]);

@@ -81,7 +81,6 @@ static int launch_conv1_inst(const paacb_ctx* ctx, const float* params, const ui
   p.batch = (int)batch;
   p.bias = params + g.b_off;
   p.wscale = ctx->wq_scale;
-  p.dbg = ctx->dbg;
   p.out_hi = out_hi;
   p.out_lo = out_lo;
   p.out_f32 = out_f32;

@@ -40,7 +40,6 @@ struct Conv1Params {
   const float* bias;
   const float* wscale;     // [NC]: s_c / (63 * 255)
   float* out_f32;          // fp32 output [b, 20, 20, NC] (F32OUT variants) instead of the planes
-  int dbg;                 // PAACB_DBG ablations (timing experiments only): 1 no stores, 2 no epilogue arithmetic, 4 no MMAs, 8 no A loads
   uint8_t* out_hi;
   uint8_t* out_lo;
   uint16_t* relu_bits;     // [b][2 planes][400 positions] uint16, plane h bit relu1_bit_pos(c) = (channel 16 h + c > 0); nullptr: not wanted (tc2.cuh)
@@ -115,7 +114,6 @@ __global__ void __launch_bounds__(C1<NC>::THREADS, 1) conv1_i8_kernel(const __gr
       uint32_t phase = 0;
       for (int tile = cta; tile < p.num_tiles; tile += ncta) {
         mbar_wait(&empty_bar[slot], phase ^ 1u);
-        if (PAACB_DBGV(p.dbg) & 8) { mbar_arrive(&full_bar[slot]); if (++slot == kC1_NSLOTS) { slot = 0; phase ^= 1u; } continue; }
         mbar_arrive_expect_tx(&full_bar[slot], kC1_BOX);
         tma_load_3d(ring + slot * kC1_SLOT, &p.tmA, 0, tile * kC1_TROWS, 0, &full_bar[slot]);
         if (++slot == kC1_NSLOTS) { slot = 0; phase ^= 1u; }
@@ -142,7 +140,7 @@ __global__ void __launch_bounds__(C1<NC>::THREADS, 1) conv1_i8_kernel(const __gr
       tc_fence_after();
       if (leader) {
 #pragma unroll
-        for (int kh = 0; kh < ((PAACB_DBGV(p.dbg) & 4) ? 1 : 8); ++kh) {           // filter row kh: parity plane kh & 3, one plane row further down for kh >= 4
+        for (int kh = 0; kh < 8; ++kh) {           // filter row kh: parity plane kh & 3, one plane row further down for kh >= 4
           const uint32_t a = ring_a + (uint32_t)(slot * kC1_SLOT + (kh & 3) * kC1_PLANE + (kh >> 2) * kC1_WU * 16);
           const uint64_t bd = desc_with_addr(bdesc0, w_a + (uint32_t)((kh / 4) * (kC1_ND * 128) + (kh % 4) * 32));
           umma_i8(d0, desc_with_addr(adesc0, a), bd, idesc, kh ? 1u : 0u);
@@ -180,10 +178,6 @@ __global__ void __launch_bounds__(C1<NC>::THREADS, 1) conv1_i8_kernel(const __gr
       uint32_t hw[8], lw[8];
       float of[F32OUT ? 16 : 1];
       const float4* sb4 = reinterpret_cast<const float4*>(s_sb) + cg * 8;
-      if (PAACB_DBGV(p.dbg) & 2) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) { hw[j] = v0[2 * j] ^ v1[2 * j + 1]; lw[j] = v2[2 * j] ^ v0[2 * j + 1]; }
-      } else
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const float4 sb = sb4[j];              // (scale, bias) of channels 2j, 2j + 1: one broadcast 16-byte load
@@ -200,7 +194,7 @@ __global__ void __launch_bounds__(C1<NC>::THREADS, 1) conv1_i8_kernel(const __gr
         if constexpr (F32OUT) { of[2 * j] = o[0]; of[2 * j + 1] = o[1]; }
         else split_bf16x2(o[0], o[1], hw[j], lw[j]);
       }
-      if (ok && !(PAACB_DBGV(p.dbg) & 1)) {                 // 16 channels = one full 32-byte sector per plane
+      if (ok) {                 // 16 channels = one full 32-byte sector per plane
         const uint32_t oh = g - n * (uint32_t)kC1_HQ;
         if constexpr (!F32OUT) {
           if (p.relu_bits != nullptr) {

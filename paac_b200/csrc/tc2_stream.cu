@@ -32,7 +32,7 @@ static int launch_stream(const paacb_ctx* ctx, const StreamParams& p, int slot, 
   const int units = p.m_tiles * p.n_tiles * p.k_splits;
   const unsigned grid = (unsigned)(units < ctx->num_sms ? units : ctx->num_sms);
   PAACB_LAUNCH_BEGIN(ctx, slot, st);
-  launch_kernel(stream_gemm_kernel<BN, MODE>, grid, kStreamThreads, Cfg::SMEM_BYTES, st, ctx->pdl_on != 0, p);
+  launch_kernel(stream_gemm_kernel<BN, MODE>, grid, kStreamThreads, Cfg::SMEM_BYTES, st, p);
   PAACB_LAUNCH_END(ctx, slot, st);
   return PAACB_OK;
 }
@@ -52,7 +52,6 @@ int launch_fc_fwd_bf16(const paacb_ctx* ctx, int l, const float* params, void* f
   if (g.K % 8 != 0 || g.N % kFcBN != 0) return PAACB_EUNSUPPORTED;
   StreamParams p;
   memset(&p, 0, sizeof(p));
-  p.dbg = ctx->dbg;
   const Planes x = layer_planes(fwd_ws, g.in_act_off, g.K, slice);
   const Planes y = layer_planes(fwd_ws, g.out_act_off, g.N, slice);
   int rc = map2d(&p.tmA[0], x.hi, (uint64_t)g.K, (uint64_t)batch, 64, 128);
@@ -80,7 +79,6 @@ int launch_fc_dgrad_bf16(const paacb_ctx* ctx, int l, const void* fwd_ws, void* 
   if (g.N % 64 != 0 || g.K % 32 != 0) return PAACB_EUNSUPPORTED;
   StreamParams p;
   memset(&p, 0, sizeof(p));
-  p.dbg = ctx->dbg;
   const Planes dz = layer_planes(bwd_ws, g.out_act_off, g.N, batch);
   const Planes dx = layer_planes(bwd_ws, gp.out_act_off, g.K, batch);
   const Planes xa = layer_planes(const_cast<void*>(fwd_ws), gp.out_act_off, g.K, batch);
@@ -110,7 +108,6 @@ int launch_fc_wgrad_bf16(const paacb_ctx* ctx, int l, const void* fwd_ws, const 
   if (g.N % kFcBN != 0 || g.K % 32 != 0) return PAACB_EUNSUPPORTED;      // ragged k-tiles: OOB columns of X read zeros
   StreamParams p;
   memset(&p, 0, sizeof(p));
-  p.dbg = ctx->dbg;
   const Planes x = layer_planes(const_cast<void*>(fwd_ws), g.in_act_off, g.K, batch);
   const Planes dz = layer_planes(const_cast<void*>(bwd_ws), g.out_act_off, g.N, batch);
   int rc = map2d(&p.tmA[0], x.hi, (uint64_t)g.K, (uint64_t)batch, 64, 64);

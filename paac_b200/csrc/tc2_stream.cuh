@@ -22,7 +22,6 @@ struct StreamParams {
   float* dbias;              // dgrad: += column sums, column c -> dbias[c % dbias_mod]
   int dbias_mod;
   float* dw;                 // wgrad target (fp32, atomics)
-  int dbg;                   // PAACB_DBG ablations (timing experiments only): 2048 no TMA loads
 };
 
 template <int BN, int MODE>
@@ -119,7 +118,6 @@ __global__ void __launch_bounds__(kStreamThreads, 1) stream_gemm_kernel(const __
         kb_range(split, kb0, kb1);
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(&empty_bar[stage], phase ^ 1u);
-          if (PAACB_DBGV(p.dbg) & 2048) { mbar_arrive(&full_bar[stage]); if (++stage == STAGES) { stage = 0; phase ^= 1u; } continue; }
           mbar_arrive_expect_tx(&full_bar[stage], Cfg::STAGE_BYTES);
           uint8_t* st = smem + stage * Cfg::STAGE_BYTES;
 #pragma unroll
@@ -213,7 +211,7 @@ __global__ void __launch_bounds__(kStreamThreads, 1) stream_gemm_kernel(const __
           const int n0 = nt * BN + c * 32;
 #pragma unroll
           for (int j = 0; j < 4; ++j) mk[c][j] = make_uint4(0u, 0u, 0u, 0u);
-          if (ok && n0 < p.N && !(PAACB_DBGV(p.dbg) & 16384)) {
+          if (ok && n0 < p.N) {
             const uint8_t* mp = p.mask_hi + ((int64_t)m * p.ldo + n0) * 2;
             ldg256(mp, mk[c][0], mk[c][1]);
             ldg256(mp + 32, mk[c][2], mk[c][3]);

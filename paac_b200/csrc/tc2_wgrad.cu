@@ -22,8 +22,8 @@ struct Wg;
 // Units are 32 B (4 pixels x 4 channels): MN groups of 16 k.  The 8 groups of a 128-row MMA are the 4 row-parity planes
 // (kh & 3; LBO = plane slot stride) for kw / 4 = 0 followed by the SAME 4 planes one unit (4 pixels) further for
 // kw / 4 = 1: the converter warps write every unit twice, into slot p and, shifted by 32 bytes, into slot p + 4, so one
-// MMA covers what were two half-empty k-tiles (the kernel is bound by its MMA count -- PAACB_DBG=128 halves it and the
-// time -- while conversion and loads are free: PAACB_DBG=64 / 32).  k-tile kt = kh / 4.
+// MMA covers what were two half-empty k-tiles (the kernel is bound by its MMA count -- half the k-tiles took half the
+// time -- while conversion and loads are free).  k-tile kt = kh / 4.
 template <>
 struct Wg<0> {
   static constexpr int A_PARTS = 8, A_PIECES = 1, A_SLOT = 9216, A_BOX = 16 * 2 * 21 * 13, B_SLOT = 16384, B_BOX = 64 * 21 * 12;
@@ -112,7 +112,6 @@ struct Wg2Params {
   const uint8_t* a_u8;    // conv1: the uint8 states [b, 84, 84, 4], converted to bf16 in shared memory, instead of tmA
   float* dw;              // [K, BN] fp32
   float w_scale;          // 1/255 for the uint8 layer (the operand holds the raw pixel values), else 1
-  int dbg;                // PAACB_DBG ablations (timing experiments only): 16 hi*hi MMAs only, 32 no TMA loads, 64 no conversion, 128 half the k-tiles
 };
 
 template <int L>
@@ -190,7 +189,6 @@ __global__ void __launch_bounds__(Wg2Cfg<L>::THREADS, 1) wgrad2_kernel(const __g
       uint32_t phase = 0;
       for (int s = s_begin; s < s_end; ++s) {
         mbar_wait(&empty_bar[stage], phase ^ 1u);
-        if (PAACB_DBGV(p.dbg) & 32) { mbar_arrive(&full_bar[stage]); if (++stage == STAGES) { stage = 0; phase ^= 1u; } continue; }
         mbar_arrive_expect_tx(&full_bar[stage], Cfg::TX_BYTES);
         uint8_t* a = a_sm + stage * Cfg::A_STAGE;
         uint8_t* b = b_sm + stage * Cfg::B_STAGE;
@@ -244,7 +242,6 @@ __global__ void __launch_bounds__(Wg2Cfg<L>::THREADS, 1) wgrad2_kernel(const __g
         const uint32_t first = (s == s_begin) ? 0u : 1u;
 #pragma unroll
         for (int kt = 0; kt < W::KT; ++kt) {
-          if ((PAACB_DBGV(p.dbg) & 128) && kt >= W::KT / 2) continue;
           const uint32_t d = tmem_base + (uint32_t)Cfg::acc_col(kt);
           const bool cat = kt < Cfg::NCAT;
           const uint64_t bdesc0 = cat ? bdesc_cat : bdesc_one;
@@ -267,10 +264,10 @@ __global__ void __launch_bounds__(Wg2Cfg<L>::THREADS, 1) wgrad2_kernel(const __g
               umma_bf16(d, desc_with_addr(adesc0, a_hi + ao), desc_with_addr(bdesc0, b_hi + bo), idesc_full, t > 0 ? 1u : first);
             } else {
               umma_bf16(d, desc_with_addr(adesc0, a_hi + ao), desc_with_addr(bdesc0, b_hi + bo), idesc, t > 0 ? 1u : first);
-              if (!(PAACB_DBGV(p.dbg) & 16)) umma_bf16(d, desc_with_addr(adesc0, a_hi + ao), desc_with_addr(bdesc0, b_lo + bo), idesc, 1u);
+              umma_bf16(d, desc_with_addr(adesc0, a_hi + ao), desc_with_addr(bdesc0, b_lo + bo), idesc, 1u);
             }
             if constexpr (W::A_PIECES == 2)
-              if (!(PAACB_DBGV(p.dbg) & 16)) umma_bf16(d, desc_with_addr(adesc0, a_lo + ao), desc_with_addr(bdesc0, b_hi + bo), idesc, 1u);
+              umma_bf16(d, desc_with_addr(adesc0, a_lo + ao), desc_with_addr(bdesc0, b_hi + bo), idesc, 1u);
           }
         }
         umma_commit(&empty_bar[stage]);
@@ -296,7 +293,7 @@ __global__ void __launch_bounds__(Wg2Cfg<L>::THREADS, 1) wgrad2_kernel(const __g
           const int w = ct + i * Cfg::CONV_THREADS;
           const int R = row0 + w / 21, u = w % 21;
           const int n = R / 21, q = R - n * 21;
-          const bool ok = (w < UNITS) && (s < s_end) && (n < p.batch) && !(PAACB_DBGV(p.dbg) & 64);
+          const bool ok = (w < UNITS) && (s < s_end) && (n < p.batch);
 #pragma unroll
           for (int part = 0; part < 4; ++part) {
             b[part][i] = make_uint4(0u, 0u, 0u, 0u);
@@ -314,7 +311,7 @@ __global__ void __launch_bounds__(Wg2Cfg<L>::THREADS, 1) wgrad2_kernel(const __g
 #pragma unroll
           for (int i = 0; i < UPT; ++i) {
             const int w = ct + i * Cfg::CONV_THREADS;
-            if (w < UNITS && !(PAACB_DBGV(p.dbg) & 64)) {
+            if (w < UNITS) {
               const uint32_t wd[4] = {b[part][i].x, b[part][i].y, b[part][i].z, b[part][i].w};
               uint32_t o[8];
 #pragma unroll
@@ -430,14 +427,10 @@ static int launch_wg2(const paacb_ctx* ctx, const Wg2Params& p, cudaStream_t st)
   }
   // multi-GPU: the gradient tail is being all-reduced while these kernels run; one persistent CTA per SM with the maximum
   // shared-memory carve-out would leave the collective's CTAs nowhere to go until a whole kernel retires
-  // (the collective is launched when the first of these kernels is: only the first sm_reserve_kernels of them -- conv3, conv2,
-  // conv1 in launch order -- leave the SMs free, PAACB_SM_RESERVE_KERNELS)
-  const int order = (ctx->n_layers - 2) - Wg<L>::LAYER;
-  const int reserve = (order < ctx->sm_reserve_kernels) ? ctx->sm_reserve : 0;
-  const int sms = ctx->num_sms - reserve > 0 ? ctx->num_sms - reserve : 1;
+  const int sms = ctx->num_sms - ctx->sm_reserve > 0 ? ctx->num_sms - ctx->sm_reserve : 1;
   const unsigned grid = (unsigned)(p.stages_total < sms ? p.stages_total : sms);
   PAACB_LAUNCH_BEGIN(ctx, K_WGRAD0 + Wg<L>::LAYER, st);
-  launch_kernel(wgrad2_kernel<L>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, st, ctx->pdl_on != 0, p);
+  launch_kernel(wgrad2_kernel<L>, grid, Cfg::THREADS, Cfg::SMEM_BYTES, st, p);
   PAACB_LAUNCH_END(ctx, K_WGRAD0 + Wg<L>::LAYER, st);
   return PAACB_OK;
 }
@@ -451,7 +444,6 @@ int launch_conv_wgrad_bf16(const paacb_ctx* ctx, int l, const uint8_t* states, c
   p.batch = (int)batch;
   p.dw = grads + g.w_off;
   p.w_scale = g.in_u8 ? 0.003921568859368563f : 1.0f;
-  p.dbg = ctx->dbg;
   const uint8_t* x_hi;
   const uint8_t* x_lo;
   if (l == 0) {

@@ -82,10 +82,11 @@ def test_large_batch_properties(net):
     assert torch.equal(out[..., 3], mx[:, row][:, :, col])
 
 
-@pytest.mark.parametrize('n', [5, 300])
+@pytest.mark.parametrize('n', [5, 120, 300])
 def test_zero_copy_from_pinned_host_frames(net, n):
     """The runners' frame buffers live in pinned, mapped host memory (Runners.pin()); the kernel reads them in place
-    (narrow grid-stride launch for n > 96).  Same bytes as with device-resident frames."""
+    (narrow grid-stride launch for 96 < n <= the SM count, the copy pipeline on 32 CTAs above it).  Same bytes as with
+    device-resident frames."""
     from paac_b200 import _lib
     rng = np.random.RandomState(100 + n)
     frames = torch.from_numpy(rng.randint(0, 256, (n, 4, 2, 210, 160)).astype(np.uint8)).pin_memory()
@@ -100,59 +101,34 @@ def test_zero_copy_from_pinned_host_frames(net, n):
     assert np.array_equal(out.cpu().numpy(), want)
 
 
-def test_planar_ring_prototype_equals_k1():
-    """SURVEY 8(f) rank 1 prototype: K1 writing only the new plane into a planar ring + the gather that rebuilds the NHWC stack
-    == K1 (bit-exact), over a ring that wraps."""
+def test_copy_pipeline_equals_cta_per_env_kernel():
+    """Device-resident frames go through the persistent copy pipeline (one CTA per SM, 4 stages) when the row table is the
+    affine default; any other table takes the CTA-per-environment kernel at the same size.  Both against the oracle, with
+    the table each was given.  1,500 environments = more than 148 x 4: every stage of the ring is refilled; 20 % of the
+    environments reset from their four pairs (out of place), and the single-pair layout runs in place."""
     import ctypes as C
-    from paac_b200 import _lib
-    N, R, steps = 33, 8, 11
-    net = G.make_net('NIPS', 4)
-    rng = np.random.RandomState(21)
-    ring = torch.zeros((N, R, 84, 84), dtype=torch.uint8, device='cuda')
-    state = np.zeros((N, 84, 84, 4), np.uint8)
-    got = torch.empty((N, 84, 84, 4), dtype=torch.uint8, device='cuda')
-    for t in range(steps):
-        frames = rng.randint(0, 256, (N, 1, 2, 210, 160)).astype(np.uint8)
-        f = G.dev(frames)
-        _lib.check(net._lib.paacb_preprocess_planar_u8(net.ctx, _lib.ptr(f), 1, _lib.ptr(ring), R, t % R, N, G.stream()), 'planar')
-        state = opre.step_states(state, frames, np.zeros(N, np.uint8), ROW, COL)
-        if t >= 3:
-            _lib.check(net._lib.paacb_stack_from_planes(net.ctx, _lib.ptr(ring), R, t % R, _lib.ptr(got), N, G.stream()), 'gather')
-            torch.cuda.synchronize()
-            assert np.array_equal(got.cpu().numpy(), state), t
-
-
-def test_copy_pipeline_equals_cta_per_env_kernel(monkeypatch):
-    """Device-resident frames go through the persistent copy pipeline (one CTA per SM, 4 stages); the CTA-per-environment
-    kernel (PAACB_K1_PIPE=0: what pinned host frames use) must write the same bytes.  1,500 environments = more than 148 x 4:
-    every stage of the ring is refilled, 20 % of the environments reset from their four pairs, in place and out of place,
-    with and without the L2 policies; 700 environments also against the oracle."""
     from paac_b200 import _lib
     n = 1500
     gen = torch.Generator(device='cuda'); gen.manual_seed(11)
     frames = torch.randint(0, 256, (n, 4, 2, 210, 160), dtype=torch.uint8, device='cuda', generator=gen)
     prev = torch.randint(0, 256, (n, 84, 84, 4), dtype=torch.uint8, device='cuda', generator=gen)
     reset = (torch.rand((n,), device='cuda', generator=gen) < 0.2).to(torch.uint8)
-    nets = {}
-    for name, env in (('pipe', {'PAACB_K1_PIPE': '1', 'PAACB_K1_HINTS': '3'}), ('pipe_nohint', {'PAACB_K1_PIPE': '1', 'PAACB_K1_HINTS': '0'}),
-                      ('cta', {'PAACB_K1_PIPE': '0'})):
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
-        nets[name] = G.make_net('NIPS', 4)
-    outs = {}
-    for name, net in nets.items():
+    assert int(reset.sum()) > 100
+    f1 = frames[:, 0].contiguous()            # single-pair layout of the same frames (pairs = 1, no resets)
+    frames_h, f1_h, prev_h, reset_h = frames.cpu().numpy(), f1[:, None].cpu().numpy(), prev.cpu().numpy(), reset.cpu().numpy()
+    row_cta = ROW.copy()
+    row_cta[5] += 1                           # breaks row(2k + 1) = row(1) + 5k: not expressible by the row-parity tensor maps
+    for name, row in (('pipeline', ROW), ('cta', row_cta)):
+        net = G.make_net('NIPS', 4)
+        r32, c32 = np.ascontiguousarray(row, np.int32), np.ascontiguousarray(COL, np.int32)
+        _lib.check(net._lib.paacb_set_resize_tables(net.ctx, r32.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                    c32.ctypes.data_as(C.POINTER(C.c_int32))), 'paacb_set_resize_tables')
         o = torch.empty_like(prev)
         _lib.check(net._lib.paacb_preprocess_u8(net.ctx, _lib.ptr(frames), 4, _lib.ptr(reset), _lib.ptr(prev), _lib.ptr(o), n, G.stream()))
-        # single-slot view of the same buffer (pairs = 1: stride of one pair, no resets), in place
-        f1 = frames[:, 0].contiguous()
         b = prev.clone()
         _lib.check(net._lib.paacb_preprocess_u8(net.ctx, _lib.ptr(f1), 1, None, _lib.ptr(b), _lib.ptr(b), n, G.stream()))
         torch.cuda.synchronize()
-        outs[name] = (o, b)
-    for name in ('pipe', 'pipe_nohint'):
-        assert torch.equal(outs[name][0], outs['cta'][0]), name
-        assert torch.equal(outs[name][1], outs['cta'][1]), name
-    assert int(reset.sum()) > 100
-    m = 700
-    want = opre.step_states(prev[:m].cpu().numpy(), frames[:m].cpu().numpy(), reset[:m].cpu().numpy(), ROW, COL)
-    assert np.array_equal(outs['pipe'][0][:m].cpu().numpy(), want)
+        want = opre.step_states(prev_h, frames_h, reset_h, row, COL)
+        assert np.array_equal(o.cpu().numpy(), want), name
+        want1 = opre.step_states(prev_h, f1_h, np.zeros(n, np.uint8), row, COL)
+        assert np.array_equal(b.cpu().numpy(), want1), name + ', one pair in place'

@@ -302,39 +302,25 @@ def test_sliced_bootstrap_equals_whole_batch():
 
 
 @pytest.mark.parametrize('b', [1, 2, 3, 37, 148 * 2 + 1, 1111])
-def test_conv3_packed_tiles_equal_input_grid_tiles(monkeypatch, b):
-    """conv3's forward with two whole samples per tile (Geo<G_FWD3P>: three patch copies, row groups at a 9-unit stride) against the
-    input-grid enumeration (PAACB_CONV3_PACKED=0): same products, same order per output row -- but the tensor core rounds a run of
-    MMAs into one accumulator differently when the run is issued in three pieces instead of one (measured: mean difference one
-    fp32 ulp), so conv1 / conv2 must be the same bits and conv3 / fc / pi / v equal to 2e-5 of their scale.  Odd batches
-    (zero-filled half tile), one tile, more tiles than SMs, a slice of a larger workspace."""
+def test_conv3_packed_tiles_vs_oracle(b):
+    """conv3's forward with two whole samples per tile (Geo<G_FWD3P>: three patch copies, row groups at a 9-unit stride), run
+    into a slice of a larger workspace, against the fp64 oracle: every layer's activations, pi and v.  Odd batches
+    (zero-filled half tile), one tile, more tiles than SMs; samples outside the slice stay untouched."""
+    A = 6
+    net = G.make_net('NATURE', A, seed=21, math='bf16x3')
+    params = network.unflatten_params(net.get_params(), 'NATURE', A)
     gen = torch.Generator(device='cuda'); gen.manual_seed(100 + b)
     states = torch.randint(0, 256, (b, 84, 84, 4), dtype=torch.uint8, device='cuda', generator=gen)
-    out = []
     cap, first = b + 5, 3
-    for knob in ('0', '1'):
-        monkeypatch.setenv('PAACB_CONV3_PACKED', knob)
-        net = G.make_net('NATURE', 6, seed=21, math='bf16x3')
-        pi = torch.full((b, 6), -1.0, device='cuda'); v = torch.full((b,), -1.0, device='cuda')
-        ws = torch.zeros((net.workspace_floats(cap),), device='cuda')
-        net.forward(states, pi, v, ws, ws_capacity=cap, ws_first=first)
-        torch.cuda.synchronize()
-        out.append((ws.view(torch.int16).clone(), pi, v))
-    w0, w1 = out[0][0], out[1][0]
-    off = 0
-    for li, e in enumerate([20 * 20 * 32, 9 * 9 * 64, 7 * 7 * 64, 512]):
-        base = off * cap * 2                    # int16 index of the layer's region: hi plane, then lo plane, e * cap each
-        if li < 2:
-            assert torch.equal(w0[base:base + 2 * e * cap], w1[base:base + 2 * e * cap]), 'layer %d' % (li + 1)
-        else:
-            def val(w):
-                hi = (w[base:base + e * cap].to(torch.int32) << 16).view(torch.float32)
-                lo = (w[base + e * cap:base + 2 * e * cap].to(torch.int32) << 16).view(torch.float32)
-                return hi.double() + lo.double()
-            v0, v1 = val(w0), val(w1)
-            assert v0.abs().max() > 0 and (v0[:first * e] == 0).all() and (v1[:first * e] == 0).all()      # outside the slice: untouched
-            assert (v0 - v1).abs().max() <= 2e-5 * v0.abs().max(), 'layer %d' % (li + 1)
-            assert ((v0 == 0) == (v1 == 0)).float().mean() > 0.999         # the same ReLU pattern up to roundings across zero
-        off += e
-    assert torch.isfinite(out[1][1]).all()
-    assert (out[0][1] - out[1][1]).abs().max() <= 1e-5 and (out[0][2] - out[1][2]).abs().max() <= 1e-5 * max(1.0, float(out[0][2].abs().max()))
+    pi = torch.full((b, A), -1.0, device='cuda'); v = torch.full((b,), -1.0, device='cuda')
+    ws = torch.zeros((net.workspace_floats(cap),), device='cuda')
+    net.forward(states, pi, v, ws, ws_capacity=cap, ws_first=first)
+    torch.cuda.synchronize()
+    ref = network.forward(params, states.cpu().numpy(), 'NATURE', dtype=torch.float64, keep=True)
+    acts = G.layer_acts(net, ws, cap)
+    for i, want in enumerate(ref['acts'] + [ref['h']]):
+        name = 'conv%d activation' % (i + 1) if i < len(ref['acts']) else 'hidden fc'
+        assert_close(acts[i][first:first + b], want.numpy(), TOL['bf16x3'], name)
+        assert not acts[i][:first].any() and not acts[i][first + b:].any(), name + ': outside the slice'
+    assert_close(pi.cpu().numpy(), ref['pi'].numpy(), TOL['bf16x3'], 'pi')
+    assert_close(v.cpu().numpy(), ref['v'].numpy(), TOL['bf16x3'], 'v')

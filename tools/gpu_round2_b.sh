@@ -1,5 +1,5 @@
 #!/bin/bash
-# round-2 GPU pass B: the two tests pass A left red, small-batch (cfg1/2/4 size), cfg5 microbench incl. the planar-ring K1 A/B,
+# round-2 GPU pass B: the two tests pass A left red, small-batch (cfg1/2/4 size), cfg5 microbench,
 # NIPS bench on the bf16x3 kernels, the ncu launch list of the default bench command
 mkdir -p gpurun_out
 timeout 900 python -m pytest tests/test_gpu_fullsize.py tests/test_gpu_update.py -m gpu -q -rA -s -p no:cacheprovider > gpurun_out/pytest_gpu_b.log 2>&1; echo "pytest rc=$?"

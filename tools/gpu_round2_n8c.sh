@@ -1,7 +1,7 @@
 #!/bin/bash
 # round 2, 8 GPUs of one box: where does the N = 8 step lose against N = 1?  The tail all-reduce on a communicator limited to the
-# reserved SMs (new default) vs NCCL's default channel count (PAACB_TAIL_MAX_CTAS=0), fewer reserving kernels, one all-reduce
-# after the whole backward; preceded by N = 1 on the same box and the 8-rank == 1-rank update check on the new default.
+# reserved SMs (new default) vs NCCL's default channel count (PAACB_TAIL_MAX_CTAS=0), one all-reduce after the whole backward;
+# preceded by N = 1 on the same box and the 8-rank == 1-rank update check on the new default.
 mkdir -p gpurun_out
 OUT=gpurun_out/r02_n8_tail_allreduce.txt
 : > $OUT
@@ -27,9 +27,8 @@ print('%-58s ms/step %.3f  value %.2f M  conv3_wgrad %.3f conv2_wgrad %.3f conv1
 PY
 PAACB_CHECK_MATH=bf16x3 timeout 200 python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29533 tools/multi_gpu_check.py 2>&1 | grep "multi_gpu_check" >> $OUT
 EXTRA=""
-run "N = 8, tail on 8 CTAs, 8 SMs reserved by 3 kernels (default)" PAACB_X=1
+run "N = 8, tail on 8 CTAs, 8 SMs reserved (default)" PAACB_X=1
 run "N = 8, tail on NCCL's default channels (round-2 behaviour)" PAACB_TAIL_MAX_CTAS=0
-run "N = 8, tail on 8 CTAs, reserved by the first kernel only" PAACB_SM_RESERVE_KERNELS=1
 EXTRA="--no_overlap_allreduce"
 run "N = 8, one all-reduce after the whole backward" PAACB_X=1
 cat $OUT

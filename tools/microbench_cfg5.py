@@ -67,21 +67,7 @@ def main():
     row('preprocess_u8 (K1)', med, best, 33936.0 * N, 83328.0 * N,
         '%d env-steps per launch; contract 33,936 B/env-step (84 rows x 160 B x 2 frames + 7,056 B new plane); the kernel '
         'also reads and rewrites the 28,224 B interleaved stack (83,328 B moved)' % N)
-    # SURVEY 8(f) rank 1, the measured A/B: K1 at its contract traffic (new plane only, planar ring of T + 3 = 8 slots) and the
-    # gather that rebuilds the NHWC stack conv1 consumes (paacb_preprocess_planar_u8 / paacb_stack_from_planes)
-    ring = torch.zeros((N, 8, 84, 84), dtype=torch.uint8, device=dev)
-    def k1p(i):
-        _lib.check(lib.paacb_preprocess_planar_u8(ctx, p(frames[i % 3]), 1, p(ring), 8, i % 8, N, st), 'k1 planar')
-    med, best = time_launches(k1p, args.iters, do_flush=False)
-    row('preprocess_planar_u8 (f1 prototype: K1 at contract traffic)', med, best, 33936.0 * N, 33936.0 * N,
-        'new 84x84 plane only into a planar ring [N, 8, 84, 84]; moves exactly the contract bytes')
-    def gather(i):
-        _lib.check(lib.paacb_stack_from_planes(ctx, p(ring), 8, i % 8, p(nxt), N, st), 'gather')
-    med, best = time_launches(gather, args.iters)
-    row('stack_from_planes (f1 prototype: planar ring -> NHWC stack)', med, best, 56448.0 * N, 56448.0 * N,
-        'reads 4 planes (28,224 B), writes the interleaved stack (28,224 B): what a planar ring adds back while conv1 consumes '
-        '16-byte (4 pixels x 4 frames) units')
-    del frames, prev, nxt, ring
+    del frames, prev, nxt
 
     # ---- K7 + K8 ----
     f = lambda *s: torch.rand(s, device=dev, generator=gen)

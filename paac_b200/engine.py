@@ -43,6 +43,7 @@ from . import _lib, parallel
 
 STATE_SHAPE = (84, 84, 4)
 FRAME_SLOT_SHAPE = (4, 2, 210, 160)
+MAX_T = 64            # kLossMaxT in csrc/loss.cu: the returns + loss kernel keeps 5 * 32 floats per time step in shared memory
 
 
 class RolloutEngine(object):
@@ -55,6 +56,9 @@ class RolloutEngine(object):
         self.ctx = network.ctx
         self.dev = network.torch_device
         self.N, self.T, self.A = int(n_envs), int(t_max), int(network.num_actions)
+        if self.T > MAX_T:
+            # refused here rather than by paacb_returns_loss_grad at the end of the first rollout
+            raise ValueError('t_max %d exceeds %d, the longest rollout the returns + loss kernel supports' % (self.T, MAX_T))
         self.B = self.N * self.T
         self.gamma, self.rho, self.eps, self.momentum = float(gamma), float(rho), float(eps), float(momentum)
         self.clip_norm = float(clip_norm)

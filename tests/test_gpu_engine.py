@@ -19,7 +19,8 @@ import gpu_util as G
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize('arch,math,A,b', [('NATURE', 'bf16x3', 6, 700), ('NIPS', 'fp32', 4, 129), ('NIPS', 'bf16x3', 18, 257)])
+@pytest.mark.parametrize('arch,math,A,b', [('NATURE', 'bf16x3', 6, 700), ('NIPS', 'fp32', 4, 129), ('NIPS', 'bf16x3', 18, 257),
+                                           ('NIPS', 'bf16x3', 9, 131)])
 def test_in_kernel_philox_sampling_matches_oracle(arch, math, A, b):
     net = G.make_net(arch, A, seed=3, math=math)
     rng_state = torch.tensor([12345, 40], dtype=torch.int64, device='cuda')
@@ -105,28 +106,34 @@ def test_observe_u8_is_preprocess_plus_bookkeeping():
 
 
 def test_rollouts_chain_without_a_copy():
-    """s_T of a rollout IS s_0 of the next (paac.py:99-112): two consecutive rollouts see one continuous state sequence."""
-    N, T, A = 8, 3, 6
-    net = G.make_net('NATURE', A, seed=3, math='bf16x3')
-    eng = RolloutEngine(net, N, T, seed=1)
-    rng = np.random.RandomState(9)
-    s = rng.randint(0, 256, (N, 84, 84, 4)).astype(np.uint8)
-    eng.state(0).copy_(G.dev(s))
-    zero = torch.zeros(N, device='cuda')
-    seq = [s]
-    for cycle in range(3):
-        first_ptr = eng.state(0).data_ptr()
-        for t in range(T):
-            eng.act(t)
-            fr = rng.randint(0, 256, (N, 1, 2, 210, 160)).astype(np.uint8)
-            eng.observe_frames(t, G.dev(fr).data_ptr(), 1, None, zero, zero)
-            torch.cuda.synchronize()
-            seq.append(opre.step_states(seq[-1], fr, np.zeros(N, np.uint8), ROW, COL))
-        assert np.array_equal(eng.get_states().cpu().numpy(), np.stack(seq[-(T + 1):]))
-        last_ptr = eng.state(T).data_ptr()
-        eng.update(0.01)
-        assert eng.state(0).data_ptr() == last_ptr and last_ptr != first_ptr
-        assert np.array_equal(eng.state(0).cpu().numpy(), seq[-1])
+    """s_T of a rollout IS s_0 of the next (paac.py:99-112): two consecutive rollouts see one continuous state sequence.
+    Step t of cycle c samples with Philox draw c * T + t: consecutive rollouts never reuse a draw."""
+    N, A, seed = 8, 6, 1
+    for T in (3, 12):                    # T = 12: each of the loss kernel's 8 warps takes more than one time step
+        net = G.make_net('NATURE', A, seed=3, math='bf16x3')
+        eng = RolloutEngine(net, N, T, seed=seed)
+        rng = np.random.RandomState(9)
+        s = rng.randint(0, 256, (N, 84, 84, 4)).astype(np.uint8)
+        eng.state(0).copy_(G.dev(s))
+        zero = torch.zeros(N, device='cuda')
+        seq = [s]
+        for cycle in range(3):
+            first_ptr = eng.state(0).data_ptr()
+            for t in range(T):
+                eng.act(t)
+                torch.cuda.synchronize()
+                u = sampling.uniforms(seed, draw=cycle * T + t, first_sample=0, count=N)
+                want = sampling.sample_actions(eng.pi_act.cpu().numpy(), u)
+                assert np.array_equal(eng.actions[t].cpu().numpy(), want), 'T %d cycle %d step %d' % (T, cycle, t)
+                fr = rng.randint(0, 256, (N, 1, 2, 210, 160)).astype(np.uint8)
+                eng.observe_frames(t, G.dev(fr).data_ptr(), 1, None, zero, zero)
+                torch.cuda.synchronize()
+                seq.append(opre.step_states(seq[-1], fr, np.zeros(N, np.uint8), ROW, COL))
+            assert np.array_equal(eng.get_states().cpu().numpy(), np.stack(seq[-(T + 1):]))
+            last_ptr = eng.state(T).data_ptr()
+            eng.update(0.01)
+            assert eng.state(0).data_ptr() == last_ptr and last_ptr != first_ptr
+            assert np.array_equal(eng.state(0).cpu().numpy(), seq[-1])
 
 
 @pytest.mark.parametrize('arch,math,mode', [('NATURE', 'bf16x3', 'batched'), ('NATURE', 'bf16x3', 'reuse'),

@@ -11,7 +11,7 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize('arch,A,b', [('NIPS', 4, 1), ('NIPS', 6, 33), ('NATURE', 6, 1), ('NATURE', 4, 7),
-                                      ('NATURE', 6, 160), ('NATURE', 18, 129), ('NIPS', 18, 160)])
+                                      ('NATURE', 6, 160), ('NATURE', 18, 129), ('NIPS', 18, 160), ('NIPS', 9, 37), ('NIPS', 2, 65)])
 def test_forward_vs_oracle(arch, A, b):
     net = G.make_net(arch, A, seed=3)
     params = network.unflatten_params(net.get_params(), arch, A)

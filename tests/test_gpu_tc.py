@@ -21,7 +21,8 @@ def skip_unsupported(math, arch):
 
 
 @pytest.mark.parametrize('math', MODES)
-@pytest.mark.parametrize('arch,A,b', [('NATURE', 6, 1), ('NATURE', 6, 130), ('NIPS', 4, 33), ('NIPS', 6, 300), ('NATURE', 18, 517)])
+@pytest.mark.parametrize('arch,A,b', [('NATURE', 6, 1), ('NATURE', 6, 130), ('NIPS', 4, 33), ('NIPS', 6, 300), ('NATURE', 18, 517),
+                                      ('NIPS', 9, 45), ('NIPS', 18, 101)])
 def test_forward_tc_vs_oracle(math, arch, A, b):
     skip_unsupported(math, arch)
     net = G.make_net(arch, A, seed=3, math=math)
@@ -39,7 +40,9 @@ def test_forward_tc_vs_oracle(math, arch, A, b):
 
 
 @pytest.mark.parametrize('math', MODES)
-@pytest.mark.parametrize('arch,A,b', [('NATURE', 6, 5), ('NATURE', 6, 160), ('NIPS', 4, 97), ('NIPS', 6, 160), ('NATURE', 4, 1111)])
+# b = 129, 257, 130: the heads backward's last 128-sample CTA holds 1 or 2 samples
+@pytest.mark.parametrize('arch,A,b', [('NATURE', 6, 5), ('NATURE', 6, 160), ('NIPS', 4, 97), ('NIPS', 6, 160), ('NATURE', 4, 1111),
+                                      ('NIPS', 9, 129), ('NIPS', 18, 257), ('NATURE', 18, 130)])
 def test_backward_tc_vs_autograd(math, arch, A, b):
     """Gradients (and every layer's dZ) against fp64 autograd whose ReLU masks are the GPU's own activations
     (oracle.network.masked_loss_and_grads): like-for-like, immune to a pre-activation rounding across zero."""
@@ -68,9 +71,12 @@ def test_auto_math_is_bf16x3_for_both_architectures():
         assert net.math == 'bf16x3' and net._lib.paacb_get_math(net.ctx) == 3
 
 
-@pytest.mark.parametrize('arch,math', [('NATURE', 'bf16x3'), ('NATURE', 'tf32x3'), ('NIPS', 'bf16x3')])
-def test_engine_update_tc_vs_oracle_composite(arch, math):
-    A, N, T = 6, 16, 5
+# T = 12 and 9: the loss kernel's warps take more than one time step each
+@pytest.mark.parametrize('arch,math,A,T', [('NATURE', 'bf16x3', 6, 5), ('NATURE', 'tf32x3', 6, 5), ('NIPS', 'bf16x3', 6, 5),
+                                          ('NIPS', 'bf16x3', 9, 12), ('NATURE', 'bf16x3', 18, 9)],
+                         ids=['NATURE-bf16x3', 'NATURE-tf32x3', 'NIPS-bf16x3', 'NIPS-bf16x3-A9-T12', 'NATURE-bf16x3-A18-T9'])
+def test_engine_update_tc_vs_oracle_composite(arch, math, A, T):
+    N = 16
     net = G.make_net(arch, A, seed=5, math=math)
     eng = RolloutEngine(net, N, T, seed=9)
     rng = np.random.RandomState(0)

@@ -16,8 +16,14 @@ import gpu_util as G
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize('T,N,A', [(5, 37, 6), (1, 1, 4), (5, 256, 18), (3, 130, 6)])
-def test_returns_loss_grad_vs_oracle(T, N, A):
+# T > 8: the kernel's 8 warps each take several time steps (t = w, w + 8, ...) and reload pi, v and the action for all but
+# the first; T = 64 is the kernel's limit (kLossMaxT)
+@pytest.mark.parametrize('T,N,A,gamma', [(5, 37, 6, 0.99), (1, 1, 4, 0.99), (5, 256, 18, 0.99), (3, 130, 6, 0.99),
+                                         (8, 33, 9, 0.99), (9, 31, 18, 0.99), (16, 100, 2, 0.99), (17, 37, 3, 0.99),
+                                         (64, 65, 9, 0.99), (9, 31, 18, 0.0), (17, 37, 3, 1.0)],
+                         ids=['5-37-6', '1-1-4', '5-256-18', '3-130-6', '8-33-9', '9-31-18', '16-100-2', '17-37-3', '64-65-9',
+                              '9-31-18-gamma0', '17-37-3-gamma1'])
+def test_returns_loss_grad_vs_oracle(T, N, A, gamma):
     net = G.make_net('NIPS', A)
     rng = np.random.RandomState(T * 1000 + N)
     rewards = rng.choice([-3.0, -1.0, 0.0, 0.5, 1.0, 7.0], size=(T, N)).astype(np.float32)
@@ -29,8 +35,8 @@ def test_returns_loss_grad_vs_oracle(T, N, A):
     logits[0, :] = [-100] * (A - 1) + [50]                      # a saturated policy row
     pi = np.exp(logits - logits.max(1, keepdims=True)); pi = (pi / pi.sum(1, keepdims=True)).astype(np.float32)
     v = rng.randn(T * N).astype(np.float32)
-    out = G.returns_loss_grad(net, rewards, over, values, boot, actions, pi, v, 0.99, 0.02)
-    y, adv = update.nstep_returns(rewards, over, values, boot, 0.99)
+    out = G.returns_loss_grad(net, rewards, over, values, boot, actions, pi, v, gamma, 0.02)
+    y, adv = update.nstep_returns(rewards, over, values, boot, gamma)
     assert np.array_equal(out['y'], y.reshape(-1)) and np.array_equal(out['adv'], adv.reshape(-1))   # f64 recurrence -> f32
     # loss / gradients: feed pi through the exact-epsilon closed form in float64 (SURVEY App. C)
     z = np.log(pi.astype(np.float64) + 1e-300)
